@@ -31,6 +31,10 @@ self-attention + heads + soft loss).
 
 `--impl reference` times the CPU path of the selected workload alone (all host threads) and prints
 the same line with "impl": "reference".
+
+`--dump-outputs DIR` writes what the timed path returned in its last step (retrieval: indices,
+values, expr_pred; cfg5: loss, dS, dI; cfg2: loss and every parameter gradient) as DIR/<name>.npy.
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -92,6 +96,38 @@ def make_inputs_device(cfg, seed, device, flavour="clustered"):
         lib = cnt.sum(1, keepdim=True).clamp_(min=1.0)
         expr[r0:r1] = torch.log10(1.0 + cnt / lib * 1e4)
     return bank, qry, expr
+
+
+# --------------------------------------------------------------------------- outputs
+DUMP_BYTES = 60 << 20          # under 64 MB whether a megabyte is 10^6 or 2^20 bytes
+
+
+def dump_outputs(dirname, arrays, seed=20261020):
+    """Writes each array of `arrays` (name -> tensor the timed path returned) as DIR/<name>.npy:
+    float32 stays float32, every other dtype becomes float64 (indices are exact in it).  All files
+    together stay within 64 MB: smallest first, an array is kept whole while it fits its share of
+    what is left; a larger one keeps a fixed, seeded sample of its rows, and the row numbers go to
+    DIR/<name>.rows.npy, so two builds run with the same arguments can be compared file by file."""
+    os.makedirs(dirname, exist_ok=True)
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a if a.dtype == np.float32 else a.astype(np.float64)
+    left = DUMP_BYTES
+    order = sorted(host, key=lambda n: host[n].nbytes)
+    for i, name in enumerate(order):
+        a = host[name]
+        share = left // (len(order) - i) - 256                 # 128-byte .npy header per file
+        if a.nbytes <= share:
+            np.save(os.path.join(dirname, name + ".npy"), a)
+            left -= a.nbytes + 128
+            continue
+        row_bytes = a.nbytes // a.shape[0] + 8                 # + its float64 row number
+        n = max(1, share // row_bytes)
+        rows = np.sort(np.random.default_rng(seed).choice(a.shape[0], n, replace=False))
+        np.save(os.path.join(dirname, name + ".npy"), a[rows])
+        np.save(os.path.join(dirname, name + ".rows.npy"), rows.astype(np.float64))
+        left -= n * row_bytes + 256
 
 
 # --------------------------------------------------------------------------- clocks
@@ -434,10 +470,12 @@ def main_loss(args, rank, world, local):
                 contrastive_loss_sharded(Sl, Il, 1.0, "soft").backward()
         else:
             Sg, Ig = S.clone().requires_grad_(True), I.clone().requires_grad_(True)
+            last = {}
 
             def step():
                 Sg.grad = Ig.grad = None
-                mloss.contrastive_loss(Sg, Ig, 1.0, "soft").backward()
+                last["loss"] = mloss.contrastive_loss(Sg, Ig, 1.0, "soft")
+                last["loss"].backward()
         quoted = B == B0
         if quoted:
             for _ in range(args.warmup):
@@ -451,6 +489,8 @@ def main_loss(args, rank, world, local):
             prof = _lib.profile_collect()
             _lib.profile_enable(False)
             clocks = clk.summary()
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, {"loss": last["loss"], "dS": Sg.grad, "dI": Ig.grad})
         else:
             ms = _time_steps(step, max(3, min(args.steps, 10)), args.warmup, dev)
         if world > 1:
@@ -738,6 +778,9 @@ def main_train(args, rank, world, local):
     gstep = GraphedTrainStep(net, batch)
     with ClockSampler(local) as clk:
         ms_graph = _time_steps(lambda: gstep(batch), args.steps, args.warmup, dev)
+    if args.dump_outputs:                     # the replay leaves the loss and every .grad in place
+        dump_outputs(args.dump_outputs, {"loss": gstep.loss, **{"grad." + n: p.grad for n, p in net.named_parameters()
+                                                                if p.grad is not None}})
     ms = ms_graph
     if world > 1:
         t = torch.tensor([ms], device=dev)
@@ -866,11 +909,18 @@ def main():
     ap.add_argument("--no-alt-grids", action="store_true", help="N > 1: skip timing the other decompositions")
     ap.add_argument("--queries", type=int, default=0, help="tuning: override the query count of the workload")
     ap.add_argument("--query-blocks", type=int, default=0, help="tuning: query blocks of the sharded pipeline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step to DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB: a fixed row sample of larger outputs)")
     args = ap.parse_args()
     assert args.warmup >= 3 or args.impl == "reference", "timing rules: W >= 3"
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the GPU path run by a single process")
     if args.workload == "cfg5":
         return main_loss(args, rank, world, local)
     if args.workload == "cfg2":
@@ -975,6 +1025,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = Q / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"indices": out[0], "values": out[1], "expr_pred": out[3]})
 
     # ---- roofline of the dominant kernel (live CUDA-event times from the timed region)
     per = {}

@@ -1,3 +1,5 @@
+import contextlib
+import hashlib
 import json
 import os
 import sys
@@ -39,6 +41,31 @@ def golden_checksum(*arrays) -> float:
         a = np.asarray(a, np.float64).ravel()
         s += float((a * (1.0 + (np.arange(a.size) % 7))).sum())
     return s
+
+
+def golden_sha256(a) -> str:
+    """Digest a golden array is stored as when the tests compare it bit for bit."""
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+@contextlib.contextmanager
+def golden_cpu_threads():
+    """One CPU thread while computing what is compared bit for bit with tests/golden/: torch's CPU
+    float32 products sum in another order when split over many threads (16 and more)."""
+    import torch
+    n = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(n)
+
+
+def golden_grad(z, key):
+    """A reference gradient stored as a fixed sample (oracle/make_golden.py::compact_model):
+    (flat indices, values, absolute maximum and L2 norm of the whole array, its shape)."""
+    return (z[key + "/idx"].astype(np.int64), z[key + "/val"], float(z[key + "/absmax"]),
+            float(z[key + "/norm"]), tuple(int(s) for s in z[key + "/shape"]))
 
 
 @pytest.fixture(scope="session")

@@ -6,7 +6,7 @@ import torch
 
 from mclstexp_b200 import loss as mloss, synth
 from oracle import oracle
-from conftest import golden_checksum
+from conftest import golden_checksum, golden_cpu_threads, golden_sha256
 from checkers import assert_grad_close, loss_closed_form_f64
 
 pytestmark = pytest.mark.gpu
@@ -44,8 +44,13 @@ def test_loss_vs_reference_golden(golden_model, case, tag):
     assert golden_checksum(S, I) == m["checksum"]
     targets = "eye" if tag == "eye" else "soft"
     scale = "mul" if tag.endswith("mul") else "div"
-    _check(S, I, m["T"], targets, scale,
-           ref=(z[f"{case}/{tag}/loss"], z[f"{case}/{tag}/dS"], z[f"{case}/{tag}/dI"]))
+    # the oracle's literal restatement is bit-equal to the reference's gradients (stored as digests)
+    with golden_cpu_threads():
+        _, dS, dI = oracle.contrastive_loss_ref(S, I, m["T"], targets, scale)
+    dS, dI = dS.numpy(), dI.numpy()
+    assert golden_sha256(dS) == str(z[f"{case}/{tag}/dS/sha256"])
+    assert golden_sha256(dI) == str(z[f"{case}/{tag}/dI/sha256"])
+    _check(S, I, m["T"], targets, scale, ref=(z[f"{case}/{tag}/loss"], dS, dI))
 
 
 @pytest.mark.parametrize("B,D,T,scale_in", [(256, 256, 1.0, 1.0), (1024, 256, 1.0, 1.0), (130, 256, 0.5, 0.3),
