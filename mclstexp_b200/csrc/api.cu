@@ -250,7 +250,7 @@ static int find_matches_stages(int stages, const float* bank, int64_t n_bank, in
                                t.q_resid, t.stats + 8, st))) return rc;
     if (stages == 1) {          // seed pass alone; the main pass follows in a second call
       prof_mark(st, "sim_seed");
-      if ((rc = launch_sim_topk(t, n_bank, n_query, top_k, nullptr, 0, st, 1, sb))) return rc;
+      if ((rc = launch_sim_topk(t, n_bank, n_query, top_k, st, 1, sb))) return rc;
       prof_mark(st, "end");
       return 0;
     }
@@ -258,7 +258,7 @@ static int find_matches_stages(int stages, const float* bank, int64_t n_bank, in
   if (n_query == 0) return 0;
   if (stages & 2) {
     prof_mark(st, "sim_topk");
-    if ((rc = launch_sim_topk(t, n_bank, n_query, top_k, nullptr, 0, st, (stages & 1) ? 0 : 2, sb))) return rc;
+    if ((rc = launch_sim_topk(t, n_bank, n_query, top_k, st, (stages & 1) ? 0 : 2, sb))) return rc;
     if (!(stages & 4)) {
       if (sb && sb->bound_k && (rc = launch_export_bound(t, n_query, top_k, sb->bound_k, sb->k_part, sb->bound_part, st))) return rc;
       prof_mark(st, "end");
@@ -266,11 +266,6 @@ static int find_matches_stages(int stages, const float* bank, int64_t n_bank, in
     }
   } else if (sb && sb->ext_bound) {
     if ((rc = launch_apply_bound(t, n_query, sb->ext_bound, st))) return rc;
-  }
-  if (sim_topk_ablate() != 0) {     // timing experiment (tuning builds only), no results
-    MCLST_CUDA(cudaMemsetAsync(out_indices, 0, (size_t)n_query * top_k * sizeof(int64_t), st));
-    prof_mark(st, "end");
-    return 0;
   }
   prof_mark(st, "rerank");
   if ((rc = launch_rerank(t, bank, n_bank, ld_bank, query, n_query, ld_query, dim, top_k,
@@ -532,5 +527,5 @@ extern "C" int mclst_debug_similarity(const float* bank, int64_t n_bank, int64_t
                              t.b_resid, t.stats, st))) return rc;
   if ((rc = launch_pack_rows(query, n_query, t.q_pad, ld_query, dim, t.nkb, t.qpack, t.q_nrm,
                              t.q_resid, t.stats + 8, st))) return rc;
-  return launch_sim_topk(t, n_bank, n_query, 1, out, ld_out, st);
+  return launch_sim_dump(t, n_bank, n_query, out, ld_out, st);
 }

@@ -17,8 +17,15 @@ int launch_exact_topk(const float* bank, int64_t N, int64_t ldb, const double* b
                       float* out_val, cudaStream_t st);
 
 // ---- tensor-core candidate path (sim_topk.cu)
+// Work decomposition of the persistent candidate kernel: W lanes (CTAs) walk closed-form unit
+// lists (sim_topk.cu: plan_lanes / lane_unit); `slots` candidate slots per query block.
+struct LanePlan {
+  int W, rounds, rest, w, R, M, Lt, slots;
+  int h, hm;      // sub-units (= fresh candidate buffers) per full-round unit / per main-lane unit
+};
 struct TcWorkspace {
-  int nkb, S, SS, cap, cluster, epw, ring, lanes;   // SS = S * (epw / 4) candidate streams per query
+  int nkb, SS, cap;         // SS = 2 * plan.slots candidate streams per query (two column halves)
+  LanePlan plan;            // of the candidate pass
   int64_t q_pad, n_pad;
   uint32_t* stats;          // [0..7] bank: max residual bits, non-finite flag; [8..15] queries
   uint8_t *qpack, *bpack;
@@ -34,7 +41,6 @@ struct TcWorkspace {
   int n_seed;
 };
 int tc_cap_for_k(int k);
-int sim_topk_ablate();   // timing experiments only: results are garbage when non-zero
 void tc_workspace(Arena& a, int64_t n_bank, int64_t n_query, int dim, int top_k, TcWorkspace& w);
 int launch_pack_rows(const float* x, int64_t rows, int64_t rows_pad, int64_t ld, int dim, int nkb,
                      uint8_t* packed, double* nrm, float* resid, uint32_t* stats, cudaStream_t st);
@@ -45,8 +51,11 @@ struct SeedBounds {
   float* bound_part;       // [Q] same for k_part rows
   const float* ext_bound;  // [Q] lower bound of the exact GLOBAL k-th best score, or null
 };
-int launch_sim_topk(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int top_k, float* dump,
-                    int64_t dump_ld, cudaStream_t st, int phase = 0, const SeedBounds* sb = nullptr);
+int launch_sim_topk(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int top_k, cudaStream_t st,
+                    int phase = 0, const SeedBounds* sb = nullptr);
+// testing aid: the raw tensor-core similarities of the packed operands into dump [n_query, dump_ld]
+int launch_sim_dump(const TcWorkspace& w, int64_t n_bank, int64_t n_query, float* dump, int64_t dump_ld,
+                    cudaStream_t st);
 int launch_apply_bound(const TcWorkspace& w, int64_t n_query, const float* ext_bound, cudaStream_t st);
 int launch_export_bound(const TcWorkspace& w, int64_t n_query, int top_k, float* bound, int k_part,
                         float* bound_part, cudaStream_t st);

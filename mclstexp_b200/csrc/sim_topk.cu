@@ -7,12 +7,12 @@
 //                  columns) per tile, K = 256.  Warp 0 streams bank slices with cp.async.bulk
 //                  (TMA engine) into a 4-stage shared-memory ring, warp 1 issues
 //                  tcgen05.mma.kind::f16 into a double-buffered 2 x 256-column TMEM
-//                  accumulator, warps 2-5 drain it with tcgen05.ld: every thread owns one
+//                  accumulator, warps 2-9 drain it with tcgen05.ld: every thread owns one
 //                  query row, compares 32 similarities per load against its running
-//                  threshold and appends the rare survivors to a per-(query, split) candidate
+//                  threshold and appends the rare survivors to a per-(query, stream) candidate
 //                  buffer in global memory (L2 resident).  The Q x N similarity matrix is
 //                  never materialised.
-//   rerank         per query: merge the splits' candidates, keep those within 2*eps of the
+//   rerank         per query: merge the streams' candidates, keep those within 2*eps of the
 //                  k-th best approximate score, recompute them exactly (fp64 accumulation of
 //                  the fp32-normalised rows), sort by (value desc, index asc), emit top-k.
 //
@@ -25,26 +25,11 @@
 // Rows for which the band overflows the candidate buffer (massive ties, pathological
 // clustering) are flagged and recomputed by the exact brute-force kernel.
 #include <algorithm>
-#include <cstdlib>
 #include "common.cuh"
 #include "retrieval.cuh"
 #include "umma.cuh"
 
 namespace mclst {
-
-// Tuning knobs (MCLST_SIM_*): read from the environment only in a tuning build
-// (-DMCLST_TUNING_KNOBS); the product library ignores them, carries only the variants it ships
-// and never calls getenv on the hot path.
-#ifdef MCLST_TUNING_KNOBS
-static int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
-}
-#define ST_ABLATE(p) ((p).ablate)
-#else
-static constexpr int env_int(const char*, int dflt) { return dflt; }
-#define ST_ABLATE(p) 0
-#endif
 
 using namespace ptx;
 
@@ -136,26 +121,41 @@ constexpr int ST_BN = 256;                      // bank rows per tile (TMEM colu
 constexpr int ST_STAGE_BYTES = 2 * TP_SLICE_BYTES;   // 256 rows x 64 halves
 constexpr int ST_A_BYTES = 4 * TP_SLICE_BYTES;       // up to 4 K slices (dim <= 256)
 constexpr int ST_SMEM = ST_A_BYTES + ST_STAGES * ST_STAGE_BYTES + 1024 /*barriers*/ + 1024 /*align*/;
+// Epilogue warps.  TMEM lanes can only be read by the warp whose id % 4 matches the lane quadrant,
+// so two warps share a quadrant and split the 256 columns of a tile between them; each (query,
+// column part) is its own candidate stream.  One epilogue warp per scheduler cannot hide its own
+// dependent-issue latency (ncu on the 4-warp version: epilogue-bound at 25 % issue utilisation).
+// Measured on B200, cfg4: 4 warps -> 34.7 ms, 8 -> 32.5 ms, 16 -> 36.4 ms (spills).
+constexpr int ST_EPW = 8;
+constexpr int ST_CP = ST_EPW / 4;               // column parts (candidate streams) per slot
+constexpr int ST_THREADS = 64 + 32 * ST_EPW;
+// At most 8 candidate streams per query (slots * ST_CP): the re-rank merges them in 16 KiB of
+// shared memory per query.
+constexpr int ST_MAX_SLOTS = 8 / ST_CP;
+
+enum class SimPass {
+  Candidates,   // the candidate pass: threshold filter into the per-(query, stream) buffers
+  Seed,         // visit a strided sample of the bank tiles, record the maximum of every 32-score chunk
+  Dump,         // testing aid: store the raw similarities
+};
 
 struct SimParams {
   const uint8_t* qpack;
   const uint8_t* bpack;
   int nkb;
   int64_t Q, N;
-  int tiles_total, S, k;
+  int tiles_total, k;
   const float* q_resid;
   const uint32_t* bank_stats;
-  uint2* cand;          // [q_pad][S * CP][CAP]  (approx score bits, bank row)
-  int* cand_cnt;        // [q_pad][S * CP]       (-1: overflow, row goes to the exact path)
+  uint2* cand;          // [q_pad][SS][CAP]  (approx score bits, bank row)
+  int* cand_cnt;        // [q_pad][SS]       (-1: overflow, row goes to the exact path)
   uint32_t* gthr;       // [q_pad] running per-query threshold shared by all streams (ordered key, 0 = none)
-  float* dump;          // debug: raw similarities [Q, dump_ld]
+  float* dump;          // Dump: raw similarities [Q, dump_ld]
   int64_t dump_ld;
-  int ablate;           // timing experiments only (MCLST_SIM_ABLATE): 1 = load TMEM but do not filter, 2 = do not even load
-  // seed pass: visit n_tiles tiles tile_begin + i * tile_stride and only record the maximum of
-  // every 32-score chunk into seed_out [q_pad][n_tiles * 8] (no candidates, no thresholds)
+  // Seed: visit n_tiles tiles tile_begin + i * tile_stride and only record the maximum of every
+  // 32-score chunk into seed_out [q_pad][n_tiles * 8] (no candidates, no thresholds)
   float* seed_out;
-  int tile_begin, tile_stride, n_tiles;     // used when seed_out != nullptr
-  int prune_gap;        // appended entries between two prunes of a row (<= CAP - 32 - survivors)
+  int tile_begin, tile_stride, n_tiles;
 };
 
 // eps: |tensor-core score - exact cosine| for a pair with fp16 residual norms rq, rs
@@ -269,9 +269,8 @@ __device__ __noinline__ PruneState warp_prune(uint2* my_buf, uint32_t* my_gthr, 
 // One 32-column chunk of one query row: append every similarity above the running threshold.
 // Two-level test (chunk max, then FILTER_GS-wide group max) keeps the common "one survivor in
 // the warp" case short; the bank-tail bound check lives in a separate (cold) instantiation.
-#ifndef FILTER_GS
-#define FILTER_GS 8
-#endif
+// Groups of 4 and 16 were measured too (DESIGN.md §3).
+constexpr int FILTER_GS = 8;
 template <int CAP, bool TAIL>
 __device__ __forceinline__ void filter_groups(const uint32_t (&v)[32], const float (&g)[32 / FILTER_GS],
                                               uint2* my_buf, int& cnt, float thr, uint32_t nb,
@@ -292,8 +291,7 @@ __device__ __forceinline__ void filter_groups(const uint32_t (&v)[32], const flo
 template <int CAP>
 __device__ __forceinline__ void filter_chunk(const uint32_t (&v)[32], uint2* my_buf,
                                              uint32_t* my_gthr, int& cnt, float& thr, int& flagged,
-                                             uint32_t nb, int n_left, int k, float e2, int& trigger,
-                                             int gap) {
+                                             uint32_t nb, int n_left, int k, float e2) {
   constexpr int NG = 32 / FILTER_GS;
   float g[NG];
 #pragma unroll
@@ -310,248 +308,31 @@ __device__ __forceinline__ void filter_chunk(const uint32_t (&v)[32], uint2* my_
     if (n_left >= 32) filter_groups<CAP, false>(v, g, my_buf, cnt, thr, nb, n_left);
     else filter_groups<CAP, true>(v, g, my_buf, cnt, thr, nb, n_left);
   }
-  // prune when the buffer is full OR `gap` entries arrived since the last prune: every prune
-  // tightens the threshold, and a tight threshold is what keeps the append path rare
-  const bool need = cnt > trigger;
+  // prune when the buffer cannot take another full chunk.  (Earlier prunes, every few appended
+  // entries, tighten the threshold sooner but were measured slower while thresholds converge.)
+  const bool need = cnt > CAP - 32;
   if (__any_sync(0xffffffffu, need)) {
     const PruneState ps = warp_prune<CAP>(my_buf, my_gthr, cnt, thr, flagged, need, k, e2);
-    if (need) trigger = min(CAP - 32, max(ps.cnt + gap, k + 16));
     cnt = ps.cnt; thr = ps.thr; flagged = ps.flagged;
   }
 }
 
-// CL  = cluster size along the query-block axis: the CL CTAs of a cluster stream the same bank
-//       tiles in lockstep; each loads 1/CL of every stage and multicasts it to all of them.
-// EPW = epilogue warps (4, 8 or 16).  TMEM lanes can only be read by the warp whose id % 4
-//       matches the lane quadrant, so EPW/4 warps share a quadrant and split the 256 columns
-//       of a tile between them; each (query, column part) is its own candidate stream.  One
-//       epilogue warp per scheduler cannot hide its own dependent-issue latency (ncu on the
-//       4-warp version: epilogue-bound at 25% issue utilisation), hence 8 by default.
-template <int CAP, int CL, int EPW>
-__global__ void __launch_bounds__(64 + 32 * EPW, 1)
-sim_topk_kernel(const SimParams p) {
-  constexpr int CP = EPW / 4;              // column parts per tile
-  constexpr int PART_COLS = ST_BN / CP;
-  constexpr int NCH = PART_COLS / 32;      // 32-column chunks per thread per tile (>= 2)
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  uint8_t* sA = smem;
-  uint8_t* sB = smem + ST_A_BYTES;
-  uint64_t* bar_full = reinterpret_cast<uint64_t*>(sB + ST_STAGES * ST_STAGE_BYTES);
-  uint64_t* bar_empty = bar_full + ST_STAGES;
-  uint64_t* bar_a = bar_empty + ST_STAGES;
-  uint64_t* bar_tfull = bar_a + 1;
-  uint64_t* bar_tempty = bar_tfull + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_tempty + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int qb = blockIdx.x, s = blockIdx.y;
-  const int nkb = p.nkb;
-  const bool seeding = p.seed_out != nullptr;
-  const int stride = seeding ? p.tile_stride : 1;
-  const int t0 = seeding ? p.tile_begin : (int)(((int64_t)p.tiles_total * s) / p.S);
-  const int t1 = seeding ? p.tile_begin + p.n_tiles * p.tile_stride
-                         : (int)(((int64_t)p.tiles_total * (s + 1)) / p.S);
-  const uint32_t crank = (CL > 1) ? cluster_ctarank() : 0u;
-  constexpr uint16_t kMask = (uint16_t)((1u << CL) - 1u);
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < ST_STAGES; ++i) { mbar_init(&bar_full[i], 1); mbar_init(&bar_empty[i], CL); }
-    mbar_init(bar_a, 1);
-    for (int i = 0; i < 2; ++i) { mbar_init(&bar_tfull[i], 1); mbar_init(&bar_tempty[i], EPW); }
-    fence_mbar_init();
-  }
-  if (warp == 1) tmem_alloc(tmem_slot, 512);
-  tc_fence_before();
-  __syncthreads();
-  if (CL > 1) cluster_sync_all();        // peers' barriers must exist before any remote signal
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ------------------------------------------------------------ TMA producer
-    if (lane == 0) {
-      const uint64_t pol_keep = policy_evict_last();
-      mbar_arrive_expect_tx(bar_a, (uint32_t)(nkb * TP_SLICE_BYTES));
-      for (int kb = 0; kb < nkb; ++kb)
-        bulk_g2s(sA + kb * TP_SLICE_BYTES,
-                 p.qpack + ((size_t)qb * nkb + kb) * TP_SLICE_BYTES, TP_SLICE_BYTES, bar_a);
-      uint32_t stage = 0, phase = 0;
-      constexpr uint32_t kShare = ST_STAGE_BYTES / CL;          // bytes this CTA fetches per stage
-      for (int t = t0; t < t1; t += stride) {
-        for (int kb = 0; kb < nkb; ++kb) {
-          mbar_wait(&bar_empty[stage], phase ^ 1);
-          mbar_arrive_expect_tx(&bar_full[stage], ST_STAGE_BYTES);
-          uint8_t* dst = sB + stage * ST_STAGE_BYTES;
-          const uint8_t* src0 = p.bpack + ((size_t)(2 * t) * nkb + kb) * TP_SLICE_BYTES;
-          const uint8_t* src1 = p.bpack + ((size_t)(2 * t + 1) * nkb + kb) * TP_SLICE_BYTES;
-          if (CL == 1) {
-            bulk_g2s_hint(dst, src0, TP_SLICE_BYTES, &bar_full[stage], pol_keep);
-            bulk_g2s_hint(dst + TP_SLICE_BYTES, src1, TP_SLICE_BYTES, &bar_full[stage], pol_keep);
-          } else {
-            // stage image = [slice of row-block 2t | slice of row-block 2t+1]; this CTA's share
-            const uint32_t off = crank * kShare;
-            const uint8_t* src = (off < (uint32_t)TP_SLICE_BYTES) ? src0 + off
-                                                                   : src1 + (off - TP_SLICE_BYTES);
-            bulk_g2s_mcast(dst + off, src, kShare, &bar_full[stage], kMask, pol_keep);
-          }
-          if (++stage == ST_STAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ------------------------------------------------------------ MMA issuer
-    if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc_f16(128, ST_BN, false);
-      mbar_wait(bar_a, 0);
-      tc_fence_after();
-      const uint32_t a_base = smem_u32(sA);
-      const uint32_t b_base = smem_u32(sB);
-      uint32_t stage = 0, phase = 0;
-      int it = 0;
-      for (int t = t0; t < t1; t += stride, ++it) {
-        const int buf = it & 1;
-        mbar_wait(&bar_tempty[buf], ((it >> 1) & 1) ^ 1);
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + buf * ST_BN;
-        for (int kb = 0; kb < nkb; ++kb) {
-          mbar_wait(&bar_full[stage], phase);
-          tc_fence_after();
-#pragma unroll
-          for (int k4 = 0; k4 < 4; ++k4) {
-            const uint64_t ad = make_smem_desc_sw128(a_base + kb * TP_SLICE_BYTES + k4 * 32);
-            const uint64_t bd = make_smem_desc_sw128(b_base + stage * ST_STAGE_BYTES + k4 * 32);
-            mma_f16_ss(d_tmem, ad, bd, idesc, (kb | k4) != 0 ? 1u : 0u);
-          }
-          if (CL == 1) mma_commit(&bar_empty[stage]);
-          else mma_commit_mcast(&bar_empty[stage], kMask);
-          if (++stage == ST_STAGES) { stage = 0; phase ^= 1; }
-        }
-        mma_commit(&bar_tfull[buf]);
-      }
-    }
-  } else {
-    // ------------------------------------------------------------ epilogue: threshold filter
-    const int quad = warp & 3;
-    const int part = (warp - 2) >> 2;
-    const int row = quad * 32 + lane;
-    const int64_t q = (int64_t)qb * 128 + row;
-    const bool q_valid = q < p.Q;
-    const int SS = p.S * CP;
-    const int stream = s * CP + part;
-    uint2* my_buf = p.cand + ((size_t)q * SS + stream) * CAP;
-    uint32_t* my_gthr = p.gthr + q;
-    const float rs_max = __uint_as_float(p.bank_stats[0]);
-    const float rq = q_valid ? p.q_resid[q] : 0.f;
-    const float e2 = 2.02f * pair_eps(rq, rs_max);
-    float thr = q_valid ? __int_as_float(0xff800000) : __int_as_float(0x7f800000);
-    int cnt = 0;
-    int flagged = 0;
-    const int k = p.k;
-    const int gap = p.prune_gap;
-    int trigger = min(CAP - 32, max(k + 16, gap + k));
-    const uint32_t t_lane = tmem_base + ((uint32_t)(quad * 32) << 16) + part * PART_COLS;
-    int it = 0;
-#pragma unroll 1
-    for (int t = t0; t < t1; t += stride, ++it) {
-      const int buf = it & 1;
-      // adopt the best threshold any other stream of this query has published so far
-      const uint32_t gk = q_valid ? *reinterpret_cast<volatile uint32_t*>(my_gthr) : 0u;
-      mbar_wait(&bar_tfull[buf], (it >> 1) & 1);
-      tc_fence_after();
-      if (gk != 0u) thr = fmaxf(thr, ord2f(gk));
-      const uint32_t taddr = t_lane + buf * ST_BN;
-      const int64_t col_base = (int64_t)t * ST_BN + part * PART_COLS;
-      const int n_valid = (int)min((int64_t)PART_COLS, p.N - col_base);   // < PART_COLS only at the bank tail
-      uint32_t va[32], vb[32];
-      if (seeding) {
-        // record the maximum of every 32-score chunk of this thread's columns
-        float* so = p.seed_out + (size_t)q * (p.n_tiles * 8) + (size_t)it * 8 + part * NCH;
-#pragma unroll 1
-        for (int c = 0; c < NCH; ++c) {
-          tmem_ld_32x32(taddr + c * 32, va);
-          tmem_ld_wait();
-          float m = -INFINITY;
-#pragma unroll
-          for (int j = 0; j < 32; ++j)
-            m = fmaxf(m, (col_base + c * 32 + j < p.N) ? __uint_as_float(va[j]) : -INFINITY);
-          if (q_valid) so[c] = m;
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&bar_tempty[buf]);
-        continue;
-      }
-      if (ST_ABLATE(p) == 2) {
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&bar_tempty[buf]);
-        continue;
-      }
-      tmem_ld_32x32(taddr, va);
-#pragma unroll 1
-      for (int c = 0; c < NCH; c += 2) {
-        tmem_ld_wait();
-        tmem_ld_32x32(taddr + (c + 1) * 32, vb);
-        if (p.dump != nullptr && q_valid) {
-          for (int j = 0; j < 32; ++j)
-            if (c * 32 + j < n_valid) p.dump[q * p.dump_ld + col_base + c * 32 + j] = __uint_as_float(va[j]);
-        }
-        if (ST_ABLATE(p) == 0)
-          filter_chunk<CAP>(va, my_buf, my_gthr, cnt, thr, flagged, (uint32_t)(col_base + c * 32),
-                            n_valid - c * 32, k, e2, trigger, gap);
-        else if ((va[0] ^ va[13] ^ va[31]) == 0x12345678u) cnt++;
-        tmem_ld_wait();
-        if (c + 2 < NCH) {
-          tmem_ld_32x32(taddr + (c + 2) * 32, va);
-        } else {
-          // this warp's columns are in registers: hand the accumulator back to the MMA warp
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bar_tempty[buf]);
-        }
-        if (p.dump != nullptr && q_valid) {
-          for (int j = 0; j < 32; ++j)
-            if ((c + 1) * 32 + j < n_valid)
-              p.dump[q * p.dump_ld + col_base + (c + 1) * 32 + j] = __uint_as_float(vb[j]);
-        }
-        if (ST_ABLATE(p) == 0)
-          filter_chunk<CAP>(vb, my_buf, my_gthr, cnt, thr, flagged,
-                            (uint32_t)(col_base + (c + 1) * 32), n_valid - (c + 1) * 32, k, e2, trigger, gap);
-        else if ((vb[0] ^ vb[13] ^ vb[31]) == 0x12345678u) cnt++;
-      }
-    }
-    if (q_valid) p.cand_cnt[(size_t)q * SS + stream] = flagged ? -1 : cnt;
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (CL > 1) cluster_sync_all();        // nobody leaves while peers may still multicast into it
-  if (warp == 1) tmem_dealloc(tmem_base, 512);
-}
-
 // ============================================================================ sim_topk (lanes)
-// Persistent form of the kernel above: one CTA ("lane") per SM walks a short list of units
-// (query block, bank-tile range, stream slot), so that every SM gets the same number of tiles
-// whatever the number of query blocks.  The (query block x stream) grid above idles SMs whenever
-// blocks * S is not close to a multiple of 148 (128 blocks on 148 SMs: 14 % lost, which is what
-// the 4x2 eight-GPU decomposition ran into) and pays for balance with extra streams per query
-// (S = 4 at 256 blocks: twice the candidates for the re-rank).  Unit lists, QT blocks, T tiles, W lanes:
+// Persistent: one CTA ("lane") per SM walks a short list of units (query block, bank-tile range,
+// candidate slot), so that every SM gets the same number of tiles whatever the number of query
+// blocks.  A (query block x stream) grid idles SMs whenever blocks * streams is not close to a
+// multiple of 148 (128 blocks on 148 SMs: 14 % lost, which is what the 4x2 eight-GPU decomposition
+// ran into) and pays for balance with extra streams per query (4 at 256 blocks: twice the
+// candidates for the re-rank).  Unit lists, QT blocks, T tiles, W lanes (LanePlan, retrieval.cuh):
 //   * rounds = QT / W full rounds: lane c takes block j*W + c over the whole bank (slot 0);
 //   * the rest = QT % W blocks share one last round of rest*T/W tiles per lane: each block gets
 //     w = W / rest dedicated lanes that split the MAIN region [0, M) of the bank w ways
 //     (slots 0..w-1), and the R = W - w*rest left-over lanes cut the TAIL region [M, T) of all
 //     rest blocks into equal linear runs (slots w, w+1), M = T*w*rest/W.
 // Lanes of a round start together and advance at the same rate, so all of them read the same
-// bank tiles at about the same time (one HBM read, the rest L2 hits) exactly like the waves of
-// the grid kernel; tail lanes take their boundary-aligned pieces first and the partial head
-// piece last for the same reason (two aligned groups instead of R unrelated streams).
-
-
-struct LanePlan {
-  int W, rounds, rest, w, R, M, Lt, slots;
-  int h, hm;      // sub-units (= fresh candidate buffers) per full-round unit / per main-lane unit
-};
+// bank tiles at about the same time (one HBM read, the rest L2 hits); tail lanes take their
+// boundary-aligned pieces first and the partial head piece last for the same reason (two aligned
+// groups instead of R unrelated streams).
 struct LaneUnit { int qb, t0, t1, slot; };
 
 __host__ __device__ inline bool lane_unit(const LanePlan& L, int T, int c, int j, LaneUnit& u) {
@@ -627,9 +408,8 @@ static LanePlan plan_lanes(int64_t qt, int64_t T, int W, int max_slots) {
   }
   // Fresh candidate buffers instead of prunes: a unit cut into h back-to-back sub-units gives each
   // its own slot, so the later ones start from the threshold the earlier ones published and rarely
-  // fill up (the grid kernel got this for free from S = 2; one long stream per query block cost
-  // 2 ms of extra prune stalls at cfg4).
-  static const int split = env_int("MCLST_SIM_ROUND_SPLIT", 2);
+  // fill up (one long stream per query block cost 2 ms of extra prune stalls at cfg4).
+  constexpr int split = 2;
   L.h = (int)std::max<int64_t>(1, std::min<int64_t>(std::min(split, max_slots), T));
   L.hm = 1;
   if (L.rest > 0) {
@@ -641,13 +421,13 @@ static LanePlan plan_lanes(int64_t qt, int64_t T, int W, int max_slots) {
   return L;
 }
 
-// SEED = true: the seed pass on the same balanced unit lists -- "tile" t of a unit is bank tile
-// tile_begin + t * tile_stride of the sample and the epilogue only records chunk maxima.
-template <int CAP, int EPW, bool SEED>
-__global__ void __launch_bounds__(64 + 32 * EPW, 1)
+// PASS (SimPass) selects what the epilogue does with the scores of a tile.  In the Seed pass
+// "tile" t of a unit is bank tile tile_begin + t * tile_stride of the sample.
+template <int CAP, SimPass PASS>
+__global__ void __launch_bounds__(ST_THREADS, 1)
 sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
-  constexpr int CP = EPW / 4;
-  constexpr int PART_COLS = ST_BN / CP;
+  constexpr bool SEED = PASS == SimPass::Seed;
+  constexpr int PART_COLS = ST_BN / ST_CP;
   constexpr int NCH = PART_COLS / 32;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -670,7 +450,7 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
     for (int i = 0; i < ST_STAGES; ++i) { mbar_init(&bar_full[i], 1); mbar_init(&bar_empty[i], 1); }
     mbar_init(bar_a, 1);
     mbar_init(bar_afree, 1);
-    for (int i = 0; i < 2; ++i) { mbar_init(&bar_tfull[i], 1); mbar_init(&bar_tempty[i], EPW); }
+    for (int i = 0; i < 2; ++i) { mbar_init(&bar_tfull[i], 1); mbar_init(&bar_tempty[i], ST_EPW); }
     fence_mbar_init();
   }
   if (warp == 1) tmem_alloc(tmem_slot, 512);
@@ -681,6 +461,8 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
 
   if (warp == 0) {
     // ------------------------------------------------------------ TMA producer
+    // Every CTA fetches its own bank slices: multicasting them across a cluster of CTAs that stream
+    // the same tiles was correct but slower on B200 (cfg4) -- L2 -> SM traffic is not the limiter.
     if (lane == 0) {
       const uint64_t pol_keep = policy_evict_last();
       uint32_t stage = 0, phase = 0;
@@ -748,13 +530,16 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
     }
   } else {
     // ------------------------------------------------------------ epilogue: threshold filter
+    // The filter runs on the warps that read TMEM.  Handing passing chunks to separate worker
+    // warps through a shared-memory event ring was bit-exact and 2 % faster once thresholds are
+    // warm (26.1 vs 26.7 ms at cfg4), but the workers fell behind while thresholds converge (38 vs
+    // 32 ms end to end).
     const int quad = warp & 3;
     const int part = (warp - 2) >> 2;
     const int row = quad * 32 + lane;
-    const int SS = L.slots * CP;
+    const int SS = L.slots * ST_CP;
     const float rs_max = __uint_as_float(p.bank_stats[0]);
     const int k = p.k;
-    const int gap = p.prune_gap;
     const uint32_t t_lane = tmem_base + ((uint32_t)(quad * 32) << 16) + part * PART_COLS;
     int it = 0;
     LaneUnit u;
@@ -762,7 +547,7 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
     for (int j = 0; lane_unit(L, T, c, j, u); ++j) {
       const int64_t q = (int64_t)u.qb * 128 + row;
       const bool q_valid = q < p.Q;
-      const int stream = u.slot * CP + part;
+      const int stream = u.slot * ST_CP + part;
       uint2* my_buf = p.cand + ((size_t)q * SS + stream) * CAP;
       uint32_t* my_gthr = p.gthr + q;
       const float rq = q_valid ? p.q_resid[q] : 0.f;
@@ -770,7 +555,6 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
       float thr = q_valid ? __int_as_float(0xff800000) : __int_as_float(0x7f800000);
       int cnt = 0;
       int flagged = 0;
-      int trigger = min(CAP - 32, max(k + 16, gap + k));
 #pragma unroll 1
       for (int t = u.t0; t < u.t1; ++t, ++it) {
         const int buf = it & 1;
@@ -783,25 +567,26 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
         const int64_t col_base = (int64_t)(SEED ? p.tile_begin + t * p.tile_stride : t) * ST_BN + part * PART_COLS;
         const int n_valid = (int)min((int64_t)PART_COLS, p.N - col_base);
         uint32_t va[32], vb[32];
-        if (SEED) {
-          // record the maximum of every 32-score chunk of this thread's columns
-          float* so = p.seed_out + (size_t)q * (p.n_tiles * 8) + (size_t)t * 8 + part * NCH;
+        if constexpr (PASS != SimPass::Candidates) {
+          // Seed: the maximum of every 32-score chunk of this thread's columns; Dump: the scores
+          float* out = SEED ? p.seed_out + (size_t)q * (p.n_tiles * 8) + (size_t)t * 8 + part * NCH
+                            : p.dump + q * p.dump_ld + col_base;
 #pragma unroll 1
           for (int ch = 0; ch < NCH; ++ch) {
             tmem_ld_32x32(taddr + ch * 32, va);
             tmem_ld_wait();
-            float m = -INFINITY;
+            if constexpr (SEED) {
+              float m = -INFINITY;
 #pragma unroll
-            for (int e = 0; e < 32; ++e)
-              m = fmaxf(m, (ch * 32 + e < n_valid) ? __uint_as_float(va[e]) : -INFINITY);
-            if (q_valid) so[ch] = m;
+              for (int e = 0; e < 32; ++e)
+                m = fmaxf(m, (ch * 32 + e < n_valid) ? __uint_as_float(va[e]) : -INFINITY);
+              if (q_valid) out[ch] = m;
+            } else if (q_valid) {
+#pragma unroll
+              for (int e = 0; e < 32; ++e)
+                if (ch * 32 + e < n_valid) out[ch * 32 + e] = __uint_as_float(va[e]);
+            }
           }
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bar_tempty[buf]);
-          continue;
-        }
-        if (ST_ABLATE(p) == 2) {
           tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(&bar_tempty[buf]);
@@ -812,336 +597,27 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
         for (int ch = 0; ch < NCH; ch += 2) {
           tmem_ld_wait();
           tmem_ld_32x32(taddr + (ch + 1) * 32, vb);
-          if (ST_ABLATE(p) == 0)
-            filter_chunk<CAP>(va, my_buf, my_gthr, cnt, thr, flagged, (uint32_t)(col_base + ch * 32),
-                              n_valid - ch * 32, k, e2, trigger, gap);
-          else if ((va[0] ^ va[13] ^ va[31]) == 0x12345678u) cnt++;
+          filter_chunk<CAP>(va, my_buf, my_gthr, cnt, thr, flagged, (uint32_t)(col_base + ch * 32),
+                            n_valid - ch * 32, k, e2);
           tmem_ld_wait();
           if (ch + 2 < NCH) {
             tmem_ld_32x32(taddr + (ch + 2) * 32, va);
           } else {
+            // this warp's columns are in registers: hand the accumulator back to the MMA warp
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(&bar_tempty[buf]);
           }
-          if (ST_ABLATE(p) == 0)
-            filter_chunk<CAP>(vb, my_buf, my_gthr, cnt, thr, flagged,
-                              (uint32_t)(col_base + (ch + 1) * 32), n_valid - (ch + 1) * 32, k, e2, trigger, gap);
-          else if ((vb[0] ^ vb[13] ^ vb[31]) == 0x12345678u) cnt++;
+          filter_chunk<CAP>(vb, my_buf, my_gthr, cnt, thr, flagged,
+                            (uint32_t)(col_base + (ch + 1) * 32), n_valid - (ch + 1) * 32, k, e2);
         }
       }
-      if (!SEED && q_valid) p.cand_cnt[(size_t)q * SS + stream] = flagged ? -1 : cnt;
+      if (PASS == SimPass::Candidates && q_valid) p.cand_cnt[(size_t)q * SS + stream] = flagged ? -1 : cnt;
     }
   }
 
   tc_fence_before();
   __syncthreads();
-  if (warp == 1) tmem_dealloc(tmem_base, 512);
-}
-
-// ============================================================================ sim_topk (event ring)
-// Same TMA -> tcgen05.mma -> TMEM pipeline, different drain.  ncu on the kernel above showed the
-// TMEM-critical warps spending half their time in single-lane append chains and L2 round trips
-// (prunes) between tcgen05.ld and the TMEM release.  Here the 8 DETECTOR warps only compute the
-// maximum of every 32-score chunk and, when it beats the row's threshold, dump the chunk
-// (8 x st.shared.v4 + header) into a shared-memory ring; 4 WORKER warps pop the records and do
-// the data-dependent part -- threshold test with all 32 lanes on the 32 scores, ballot
-// compaction, append, prune -- off the TMEM critical path.  A row is always handled by worker
-// (row % 4), so its candidate buffer, count and threshold have a single writer, and the two
-// column halves of a row share one stream (streams per query = S, not 2 S).
-constexpr int RG_DET = 8;                 // detector warps (2 per TMEM lane quadrant)
-constexpr int RG_WRK = 4;                 // worker warps
-constexpr int RG_THREADS = 64 + 32 * (RG_DET + RG_WRK);
-constexpr int RG_SLOTS = 44;              // records per worker ring
-constexpr int RG_REC_WORDS = 36;          // 32 scores + row + column base + 2 pad  (144 B)
-constexpr int RG_EXTRA = RG_WRK * RG_SLOTS * (RG_REC_WORDS + 1) * 4 + 128 * 16 + 256;
-constexpr int RG_SMEM = ST_A_BYTES + ST_STAGES * ST_STAGE_BYTES + 1024 + RG_EXTRA + 1024;
-static_assert(RG_SMEM <= 232448, "ring kernel exceeds the 227 KiB shared-memory limit");
-
-template <int CAP>
-__global__ void __launch_bounds__(RG_THREADS, 1)
-sim_topk_ring_kernel(const SimParams p) {
-  constexpr int PART_COLS = ST_BN / 2;
-  constexpr int NCH = PART_COLS / 32;
-  constexpr int EPL = CAP / 32;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  uint8_t* sA = smem;
-  uint8_t* sB = smem + ST_A_BYTES;
-  uint64_t* bar_full = reinterpret_cast<uint64_t*>(sB + ST_STAGES * ST_STAGE_BYTES);
-  uint64_t* bar_empty = bar_full + ST_STAGES;
-  uint64_t* bar_a = bar_empty + ST_STAGES;
-  uint64_t* bar_tfull = bar_a + 1;
-  uint64_t* bar_tempty = bar_tfull + 2;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_tempty + 2);
-  // ---- ring + per-row state (after the 1 KiB barrier block)
-  uint32_t* ring = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(bar_full) + 1024);
-  volatile int* ring_seq = reinterpret_cast<volatile int*>(ring + RG_WRK * RG_SLOTS * RG_REC_WORDS);
-  uint32_t* thr_sm = const_cast<uint32_t*>(reinterpret_cast<volatile uint32_t*>(ring_seq + RG_WRK * RG_SLOTS));
-  int* cnt_sm = reinterpret_cast<int*>(thr_sm + 128);
-  float* e2_sm = reinterpret_cast<float*>(cnt_sm + 128);
-  int* flag_sm = reinterpret_cast<int*>(e2_sm + 128);
-  int* ring_head = flag_sm + 128;                  // [RG_WRK] reserved records
-  volatile int* ring_tail = ring_head + RG_WRK;    // [RG_WRK] consumed records
-  int* det_done = const_cast<int*>(ring_tail) + RG_WRK;
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int qb = blockIdx.x, s = blockIdx.y;
-  const int nkb = p.nkb;
-  const int t0 = (int)(((int64_t)p.tiles_total * s) / p.S);
-  const int t1 = (int)(((int64_t)p.tiles_total * (s + 1)) / p.S);
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < ST_STAGES; ++i) { mbar_init(&bar_full[i], 1); mbar_init(&bar_empty[i], 1); }
-    mbar_init(bar_a, 1);
-    for (int i = 0; i < 2; ++i) { mbar_init(&bar_tfull[i], 1); mbar_init(&bar_tempty[i], RG_DET); }
-    fence_mbar_init();
-  }
-  for (int i = threadIdx.x; i < RG_WRK * RG_SLOTS; i += RG_THREADS) ring_seq[i] = 0;
-  if (threadIdx.x < 128) {
-    const int64_t q = (int64_t)qb * 128 + threadIdx.x;
-    const bool ok = q < p.Q;
-    const float rs_max = __uint_as_float(p.bank_stats[0]);
-    e2_sm[threadIdx.x] = 2.02f * pair_eps(ok ? p.q_resid[q] : 0.f, rs_max);
-    const uint32_t g = ok ? p.gthr[q] : 0u;
-    // ordered key of the threshold: -inf for live rows, +inf for padding rows (never pass)
-    thr_sm[threadIdx.x] = ok ? (g != 0u ? g : f2ord(__int_as_float(0xff800000)))
-                             : f2ord(__int_as_float(0x7f800000));
-    cnt_sm[threadIdx.x] = 0;
-    flag_sm[threadIdx.x] = 0;
-  }
-  if (threadIdx.x < RG_WRK) { ring_head[threadIdx.x] = 0; ring_tail[threadIdx.x] = 0; }
-  if (threadIdx.x == 0) *det_done = 0;
-  if (warp == 1) tmem_alloc(tmem_slot, 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ------------------------------------------------------------ TMA producer
-    if (lane == 0) {
-      const uint64_t pol_keep = policy_evict_last();
-      mbar_arrive_expect_tx(bar_a, (uint32_t)(nkb * TP_SLICE_BYTES));
-      for (int kb = 0; kb < nkb; ++kb)
-        bulk_g2s(sA + kb * TP_SLICE_BYTES,
-                 p.qpack + ((size_t)qb * nkb + kb) * TP_SLICE_BYTES, TP_SLICE_BYTES, bar_a);
-      uint32_t stage = 0, phase = 0;
-      for (int t = t0; t < t1; ++t) {
-        for (int kb = 0; kb < nkb; ++kb) {
-          mbar_wait(&bar_empty[stage], phase ^ 1);
-          mbar_arrive_expect_tx(&bar_full[stage], ST_STAGE_BYTES);
-          uint8_t* dst = sB + stage * ST_STAGE_BYTES;
-          bulk_g2s_hint(dst, p.bpack + ((size_t)(2 * t) * nkb + kb) * TP_SLICE_BYTES, TP_SLICE_BYTES,
-                        &bar_full[stage], pol_keep);
-          bulk_g2s_hint(dst + TP_SLICE_BYTES, p.bpack + ((size_t)(2 * t + 1) * nkb + kb) * TP_SLICE_BYTES,
-                        TP_SLICE_BYTES, &bar_full[stage], pol_keep);
-          if (++stage == ST_STAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ------------------------------------------------------------ MMA issuer
-    if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc_f16(128, ST_BN, false);
-      mbar_wait(bar_a, 0);
-      tc_fence_after();
-      const uint32_t a_base = smem_u32(sA);
-      const uint32_t b_base = smem_u32(sB);
-      uint32_t stage = 0, phase = 0;
-      int it = 0;
-      for (int t = t0; t < t1; ++t, ++it) {
-        const int buf = it & 1;
-        mbar_wait(&bar_tempty[buf], ((it >> 1) & 1) ^ 1);
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + buf * ST_BN;
-        for (int kb = 0; kb < nkb; ++kb) {
-          mbar_wait(&bar_full[stage], phase);
-          tc_fence_after();
-#pragma unroll
-          for (int k4 = 0; k4 < 4; ++k4) {
-            const uint64_t ad = make_smem_desc_sw128(a_base + kb * TP_SLICE_BYTES + k4 * 32);
-            const uint64_t bd = make_smem_desc_sw128(b_base + stage * ST_STAGE_BYTES + k4 * 32);
-            mma_f16_ss(d_tmem, ad, bd, idesc, (kb | k4) != 0 ? 1u : 0u);
-          }
-          mma_commit(&bar_empty[stage]);
-          if (++stage == ST_STAGES) { stage = 0; phase ^= 1; }
-        }
-        mma_commit(&bar_tfull[buf]);
-      }
-    }
-  } else if (warp < 2 + RG_DET) {
-    // ------------------------------------------------------------ detectors
-    const int quad = warp & 3;
-    const int part = (warp - 2) >> 2;
-    const int row = quad * 32 + lane;
-    const int64_t q = (int64_t)qb * 128 + row;
-    const bool q_valid = q < p.Q;
-    const int wk = row & (RG_WRK - 1);
-    uint32_t* my_ring = ring + wk * RG_SLOTS * RG_REC_WORDS;
-    volatile int* my_seq = ring_seq + wk * RG_SLOTS;
-    const uint32_t t_lane = tmem_base + ((uint32_t)(quad * 32) << 16) + part * PART_COLS;
-    int it = 0;
-#pragma unroll 1
-    for (int t = t0; t < t1; ++t, ++it) {
-      const int buf = it & 1;
-      // another CTA / stream of this query may have published a better bound
-      const uint32_t gk = q_valid ? *reinterpret_cast<volatile uint32_t*>(p.gthr + q) : 0u;
-      mbar_wait(&bar_tfull[buf], (it >> 1) & 1);
-      tc_fence_after();
-      uint32_t tk = *reinterpret_cast<volatile uint32_t*>(thr_sm + row);
-      if (gk > tk) { atomicMax(thr_sm + row, gk); tk = gk; }
-      const float thr = ord2f(tk);
-      const uint32_t taddr = t_lane + buf * ST_BN;
-      const uint32_t col_base = (uint32_t)t * ST_BN + part * PART_COLS;
-      uint32_t va[32], vb[32];
-      tmem_ld_32x32(taddr, va);
-#pragma unroll 1
-      for (int c = 0; c < NCH; c += 2) {
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          uint32_t (&v)[32] = h ? vb : va;
-          tmem_ld_wait();
-          if (h == 0) {
-            tmem_ld_32x32(taddr + (c + 1) * 32, vb);
-          } else if (c + 2 < NCH) {
-            tmem_ld_32x32(taddr + (c + 2) * 32, va);
-          } else {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&bar_tempty[buf]);
-          }
-          if (p.dump != nullptr && q_valid) {
-            for (int j = 0; j < 32; ++j) {
-              const int64_t col = (int64_t)col_base + (c + h) * 32 + j;
-              if (col < p.N) p.dump[q * p.dump_ld + col] = __uint_as_float(v[j]);
-            }
-          }
-          float m = __uint_as_float(v[0]);
-#pragma unroll
-          for (int j = 1; j < 32; ++j) m = fmaxf(m, __uint_as_float(v[j]));
-          if (ST_ABLATE(p) == 0 && m > thr) {
-            // hand the chunk to the row's worker
-            const int slot = atomicAdd(&ring_head[wk], 1);
-            if (slot - ring_tail[wk] >= RG_SLOTS) {
-              const uint64_t w0 = globaltimer();
-              while (slot - ring_tail[wk] >= RG_SLOTS)
-                if (globaltimer() - w0 > 4000000000ull) __trap();
-            }
-            uint32_t* rec = my_ring + (slot % RG_SLOTS) * RG_REC_WORDS;
-#pragma unroll
-            for (int j = 0; j < 32; j += 4)
-              *reinterpret_cast<uint4*>(rec + j) = make_uint4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-            rec[32] = (uint32_t)row;
-            rec[33] = col_base + (c + h) * 32;
-            __threadfence_block();
-            my_seq[slot % RG_SLOTS] = slot + 1;
-          }
-        }
-      }
-    }
-    __syncwarp();
-    if (lane == 0) { __threadfence_block(); atomicAdd(det_done, 1); }
-  } else {
-    // ------------------------------------------------------------ workers
-    const int wk = warp - (2 + RG_DET);
-    const uint32_t* my_ring = ring + wk * RG_SLOTS * RG_REC_WORDS;
-    volatile int* my_seq = ring_seq + wk * RG_SLOTS;
-    const int k = p.k;
-    int t = 0;
-    for (;;) {
-      // wait for record t (or for the detectors to finish with nothing left)
-      bool have = false;
-      uint32_t spins = 0;
-      const uint64_t w_start = globaltimer();
-      for (;;) {
-        if (my_seq[t % RG_SLOTS] == t + 1) { have = true; break; }
-        if (*reinterpret_cast<volatile int*>(det_done) == RG_DET &&
-            *reinterpret_cast<volatile int*>(&ring_head[wk]) == t) break;
-        if ((++spins & 0xfffu) == 0 && globaltimer() - w_start > 20000000000ull) __trap();
-      }
-      if (!have) break;
-      __threadfence_block();
-      const uint32_t* rec = my_ring + (t % RG_SLOTS) * RG_REC_WORDS;
-      const uint32_t vbits = rec[lane];
-      const int row = (int)rec[32];
-      const uint32_t cb = rec[33];
-      __syncwarp();
-      if (lane == 0) ring_tail[wk] = t + 1;          // the slot may be reused
-      ++t;
-      const float v = __uint_as_float(vbits);
-      const float thr = ord2f(*reinterpret_cast<volatile uint32_t*>(thr_sm + row));
-      const bool pass = v > thr && (int64_t)cb + lane < p.N;
-      const unsigned bal = __ballot_sync(0xffffffffu, pass);
-      if (bal == 0u) continue;
-      const int64_t q = (int64_t)qb * 128 + row;
-      uint2* buf = p.cand + ((size_t)q * p.S + s) * CAP;
-      int cnt = cnt_sm[row];
-      if (pass) buf[cnt + __popc(bal & ((1u << lane) - 1u))] = make_uint2(vbits, cb + lane);
-      cnt += __popc(bal);
-      if (cnt > CAP - 32) {
-        // ---- prune the row: threshold = (lower bound of its k-th best) - e2
-        __syncwarp();
-        __threadfence_block();
-        uint32_t keys[EPL], vals[EPL], idxs[EPL];
-#pragma unroll
-        for (int j = 0; j < EPL; ++j) {
-          const int i = lane + 32 * j;
-          if (i < cnt) {
-            const uint2 e = buf[i];
-            vals[j] = e.x; idxs[j] = e.y; keys[j] = f2ord(__uint_as_float(e.x));
-          } else {
-            keys[j] = 0u; vals[j] = 0u; idxs[j] = 0u;
-          }
-        }
-        uint32_t T = 0;
-#pragma unroll 1
-        for (int bit = 31; bit >= 8; --bit) {
-          const uint32_t cand = T | (1u << bit);
-          int c = 0;
-#pragma unroll
-          for (int j = 0; j < EPL; ++j) c += (keys[j] >= cand) ? 1 : 0;
-          c = __reduce_add_sync(0xffffffffu, c);
-          if (c >= k) T = cand;
-        }
-        float new_thr = ord2f(T) - e2_sm[row];
-        uint32_t nk = f2ord(new_thr);
-        if (lane == 0) {
-          const uint32_t old = atomicMax(p.gthr + q, nk);     // publish; adopt a better global bound
-          if (old > nk) nk = old;
-        }
-        nk = __shfl_sync(0xffffffffu, nk, 0);
-        new_thr = ord2f(nk);
-        int out = 0;
-#pragma unroll
-        for (int j = 0; j < EPL; ++j) {
-          const int i = lane + 32 * j;
-          const bool keep = (i < cnt) && (__uint_as_float(vals[j]) > new_thr);
-          const unsigned b2 = __ballot_sync(0xffffffffu, keep);
-          if (keep) buf[out + __popc(b2 & ((1u << lane) - 1u))] = make_uint2(vals[j], idxs[j]);
-          out += __popc(b2);
-        }
-        cnt = out;
-        if (lane == 0) {
-          if (out > CAP - 64) {            // band denser than the buffer: exact path takes the row
-            flag_sm[row] = 1;
-            atomicMax(thr_sm + row, f2ord(__int_as_float(0x7f800000)));
-          } else {
-            atomicMax(thr_sm + row, nk);
-          }
-        }
-      }
-      if (lane == 0) cnt_sm[row] = cnt;
-      __syncwarp();
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (threadIdx.x < 128) {
-    const int64_t q = (int64_t)qb * 128 + threadIdx.x;
-    if (q < p.Q) p.cand_cnt[(size_t)q * p.S + s] = flag_sm[threadIdx.x] ? -1 : cnt_sm[threadIdx.x];
-  }
   if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
@@ -1356,9 +832,7 @@ __device__ __forceinline__ double row_dot(const float* __restrict__ sp, const do
   return acc;
 }
 
-#ifndef RR_MIN_BLOCKS
-#define RR_MIN_BLOCKS 4      // 5 (96 registers, 140 B of spills) measured equal: latency is hidden by the 4x unrolled loads
-#endif
+constexpr int RR_MIN_BLOCKS = 4;   // 5 (96 registers, 140 B of spills) measured equal: latency is hidden by the 4x unrolled loads
 template <bool VEC, bool WANT_L1>
 __global__ void __launch_bounds__(128, RR_MIN_BLOCKS)
 rerank_kernel(const RerankParams p, int warps_per_block, int per_warp_entries) {
@@ -1581,82 +1055,15 @@ rerank_kernel(const RerankParams p, int warps_per_block, int per_warp_entries) {
 }
 
 // ============================================================================ host side
-int sim_topk_epw();
-int sim_topk_use_lanes();
-int sim_topk_cluster(int64_t n_query) {
-  static const int forced = env_int("MCLST_SIM_CLUSTER", 0);
-  if (forced == 1 || forced == 2 || forced == 4) return forced;
-  (void)n_query;
-  return 1;        // measured on B200 (cfg4): multicast clusters do not pay (L2 is not the limiter)
-}
-
-int sim_topk_ablate() {
-  static const int v = env_int("MCLST_SIM_ABLATE", 0);
-  return v;
-}
-bool sim_topk_tuning_build() {
-#ifdef MCLST_TUNING_KNOBS
-  return true;
-#else
-  return false;
-#endif
-}
-
-int sim_topk_use_ring() {
-  // Event-ring drain (sim_topk_ring_kernel): bit-exact and 2 % faster than the per-thread drain
-  // once thresholds are warm (26.1 vs 26.7 ms at cfg4), but its 4 worker warps fall behind while
-  // thresholds are still converging (38 vs 32 ms end to end) -- off until the seed pass is tighter.
-  static const int v = env_int("MCLST_SIM_RING", 0);
-  return v;
-}
-
-int sim_topk_use_lanes() {
-  // persistent lane kernel (balanced unit lists) instead of the (query block x stream) grid
-  static const int v = env_int("MCLST_SIM_LANES", 1);
-  return v;
-}
-
-int sim_topk_epw() {
-  static const int forced = env_int("MCLST_SIM_EPW", 0);
-  if (forced == 4 || forced == 8 || forced == 16) return forced;
-  return 8;      // measured on B200, cfg4: 4 -> 34.7 ms, 8 -> 32.5 ms, 16 -> 36.4 ms
-}
-
-int sim_topk_splits(int64_t n_query, int64_t n_bank, int cluster) {
-  static const int forced = env_int("MCLST_SIM_SPLITS", 0);
-  const int sms = sm_count();
-  const int64_t qblocks = ceil_div(ceil_div(n_query, 128), cluster) * cluster;
-  const int64_t tiles = ceil_div(n_bank, ST_BN);
-  if (forced > 0) return (int)std::min<int64_t>(forced, tiles);
-  int best = 1;
-  double best_eff = 0.0;
-  // at most 8 candidate streams per query (S * epw/4): the re-rank merges them in 16 KiB of
-  // shared memory per query
-  const int smax = (int)std::min<int64_t>(sim_topk_use_ring() ? 8 : std::max(1, 8 / (sim_topk_epw() / 4)), tiles);
-  for (int S = 1; S <= smax; ++S) {
-    const int64_t ctas = qblocks * S;
-    const double eff = (double)ctas / (double)(ceil_div(ctas, sms) * sms);
-    if (eff > best_eff * 1.02) { best_eff = eff; best = S; }
-  }
-  return best;
-}
-
 int tc_cap_for_k(int k) { return k <= 192 ? 256 : (k <= 896 ? 1024 : 0); }
 
 void tc_workspace(Arena& a, int64_t n_bank, int64_t n_query, int dim, int top_k, TcWorkspace& w) {
   const int nkb = (dim + 63) / 64;
   w.nkb = nkb;
-  w.cluster = sim_topk_cluster(n_query);
-  w.epw = sim_topk_epw();
-  if (tc_cap_for_k(top_k) == 1024 && w.epw == 16) w.epw = 8;   // only <1024, *, {4,8}> is built
-  w.q_pad = (int64_t)align_up((size_t)n_query, 128 * w.cluster);
+  w.q_pad = (int64_t)align_up((size_t)n_query, 128);
   w.n_pad = (int64_t)align_up((size_t)n_bank, ST_BN);
-  w.S = sim_topk_splits(n_query, n_bank, w.cluster);
-  w.ring = sim_topk_use_ring() && w.cluster == 1 && tc_cap_for_k(top_k) <= 512;
-  w.lanes = sim_topk_use_lanes() && !w.ring && w.cluster == 1;
-  if (w.lanes)
-    w.S = plan_lanes(w.q_pad / 128, w.n_pad / ST_BN, sm_count(), std::max(1, 8 / (w.epw / 4))).slots;
-  w.SS = w.ring ? w.S : w.S * (w.epw / 4);
+  w.plan = plan_lanes(w.q_pad / 128, w.n_pad / ST_BN, sm_count(), ST_MAX_SLOTS);
+  w.SS = w.plan.slots * ST_CP;
   w.cap = tc_cap_for_k(top_k);
   // everything derived from the bank first: its offsets do not depend on the query count, so a
   // resident bank (MCLST_FM_BANK_PACKED) stays valid across calls with different query batches
@@ -1678,10 +1085,8 @@ void tc_workspace(Arena& a, int64_t n_bank, int64_t n_query, int dim, int top_k,
   // seed pass 1.41 -> 1.04 ms but main pass 13.5 -> 14.7 ms at 500k rows -- the looser start costs
   // more than the sample saves.
   const int64_t tiles = w.n_pad / ST_BN;
-  static const int seed_max = env_int("MCLST_SIM_SEED_TILES", 128);
-  int n_seed = (int)std::min<int64_t>(seed_max, tiles / 8);
-  static const int seed_env = env_int("MCLST_SIM_SEED", 1);
-  if (!seed_env || n_seed * 8 < 2 * top_k) n_seed = 0;
+  int n_seed = (int)std::min<int64_t>(128, tiles / 8);
+  if (n_seed * 8 < 2 * top_k) n_seed = 0;
   w.n_seed = n_seed;
   w.seed = n_seed ? a.take<float>((size_t)w.q_pad * n_seed * 8) : nullptr;
 }
@@ -1697,41 +1102,22 @@ int launch_pack_rows(const float* x, int64_t rows, int64_t rows_pad, int64_t ld,
   return 0;
 }
 
-template <int CAP, int CL, int EPW>
-static int launch_sim_topk_t(const SimParams& p, dim3 grid, cudaStream_t st) {
-  auto kern = sim_topk_kernel<CAP, CL, EPW>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    MCLST_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM));
-    attr_set = true;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(64 + 32 * EPW);
-  cfg.dynamicSmemBytes = ST_SMEM;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  MCLST_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
+template <int CAP, SimPass PASS>
+static int launch_lanes(const SimParams& p, const LanePlan& L, cudaStream_t st) {
+  auto kern = sim_topk_lanes_kernel<CAP, PASS>;
+  MCLST_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM));
+  kern<<<(unsigned)L.W, ST_THREADS, ST_SMEM, st>>>(p, L);
   MCLST_LAUNCH_CHECK();
   return 0;
 }
 
-template <int CAP, int CL>
-static int launch_sim_topk_e(int epw, const SimParams& p, dim3 grid, cudaStream_t st) {
-  switch (epw) {
-#ifdef MCLST_TUNING_KNOBS
-    case 4: return launch_sim_topk_t<CAP, CL, 4>(p, grid, st);
-    case 16: return launch_sim_topk_t<CAP, CL, 16>(p, grid, st);
-#endif
-    case 8: return launch_sim_topk_t<CAP, CL, 8>(p, grid, st);
-  }
-  MCLST_REQUIRE(false, MCLST_ERR_UNSUPPORTED, "sim_topk: epilogue warps %d", epw);
+static SimParams sim_params(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int top_k) {
+  SimParams p{};
+  p.qpack = w.qpack; p.bpack = w.bpack; p.nkb = w.nkb; p.Q = n_query; p.N = n_bank;
+  p.tiles_total = (int)(w.n_pad / ST_BN); p.k = top_k;
+  p.q_resid = w.q_resid; p.bank_stats = w.stats; p.cand = w.cand; p.cand_cnt = w.cand_cnt;
+  p.gthr = w.gthr;
+  return p;
 }
 
 // Speculative warm start.  The guaranteed seed threshold is the k-th largest value of the sample
@@ -1759,23 +1145,13 @@ int spec_rank(int k, double f) {
   return std::max(4, std::min(best, k));
 }
 
-int launch_sim_topk(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int top_k, float* dump,
-                    int64_t dump_ld, cudaStream_t st, int phase, const SeedBounds* sb) {
+int launch_sim_topk(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int top_k, cudaStream_t st,
+                    int phase, const SeedBounds* sb) {
   // phase 0: seed pass + main pass; 1: thresholds reset + seed pass only (optionally writing the
   // cross-shard bounds of sb); 2: main pass only, after applying sb->ext_bound when given
-  SimParams p;
-  p.qpack = w.qpack; p.bpack = w.bpack; p.nkb = w.nkb; p.Q = n_query; p.N = n_bank;
-  p.tiles_total = (int)(w.n_pad / ST_BN); p.S = w.S; p.k = top_k;
-  p.q_resid = w.q_resid; p.bank_stats = w.stats; p.cand = w.cand; p.cand_cnt = w.cand_cnt;
-  p.gthr = w.gthr; p.dump = dump; p.dump_ld = dump_ld;
-  p.ablate = sim_topk_ablate();
-  p.seed_out = nullptr; p.tile_begin = 0; p.tile_stride = 1; p.n_tiles = 0;
-  static const int gap_env = env_int("MCLST_SIM_PRUNE_GAP", 1 << 20);
-  p.prune_gap = gap_env;
-  static const int keep_gthr = env_int("MCLST_SIM_KEEP_GTHR", 0);   // experiment: warm thresholds
-  if (!keep_gthr && phase != 2) MCLST_CUDA(cudaMemsetAsync(w.gthr, 0, (size_t)w.q_pad * sizeof(uint32_t), st));
-  dim3 grid((unsigned)(w.q_pad / 128), (unsigned)w.S);
-  const bool seeded = w.n_seed > 0 && dump == nullptr && !keep_gthr && p.ablate == 0;
+  const SimParams p = sim_params(w, n_bank, n_query, top_k);
+  if (phase != 2) MCLST_CUDA(cudaMemsetAsync(w.gthr, 0, (size_t)w.q_pad * sizeof(uint32_t), st));
+  const bool seeded = w.n_seed > 0;
   if (phase == 1 && !seeded && sb) {       // no sample: no bound to offer
     if (sb->bound_k) fill_kernel<<<(unsigned)ceil_div(n_query, 256), 256, 0, st>>>(sb->bound_k, n_query, -INFINITY);
     if (sb->bound_part) fill_kernel<<<(unsigned)ceil_div(n_query, 256), 256, 0, st>>>(sb->bound_part, n_query, -INFINITY);
@@ -1787,26 +1163,14 @@ int launch_sim_topk(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int t
     MCLST_LAUNCH_CHECK();
   }
   if (seeded && phase != 2) {
-    // ---- seed pass (legacy drain, 8 epilogue warps, one CTA per query block)
+    // ---- seed pass, on balanced unit lists of its own over the sampled tiles
     SimParams sp = p;
     sp.seed_out = w.seed; sp.n_tiles = w.n_seed; sp.tile_begin = 0;
     sp.tile_stride = std::max(1, p.tiles_total / w.n_seed);
-    sp.S = 1;
-    if (w.lanes) {
-      // balanced persistent form; one sub-unit per unit (no candidate slots involved)
-      LanePlan SL = plan_lanes(w.q_pad / 128, w.n_seed, sm_count(), 4);
-      auto kern = sim_topk_lanes_kernel<256, 8, true>;
-      MCLST_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM));
-      kern<<<(unsigned)SL.W, 64 + 32 * 8, ST_SMEM, st>>>(sp, SL);
-      MCLST_LAUNCH_CHECK();
-    } else {
-      dim3 sgrid((unsigned)(w.q_pad / 128), 1);
-      int rc = launch_sim_topk_t<256, 1, 8>(sp, sgrid, st);
-      if (rc) return rc;
-    }
+    int rc = launch_lanes<256, SimPass::Seed>(sp, plan_lanes(w.q_pad / 128, w.n_seed, sm_count(), 4), st);
+    if (rc) return rc;
     // bounds that other shards will rely on must be guaranteed ones: no speculation when staged
-    static const int spec_env = env_int("MCLST_SIM_SPEC", 1);
-    const bool speculate = w.speculate && spec_env && !(sb && (sb->bound_k || sb->bound_part));
+    const bool speculate = w.speculate && !(sb && (sb->bound_k || sb->bound_part));
     const int k_seed = speculate ? spec_rank(top_k, (double)w.n_seed / (double)p.tiles_total) : top_k;
     seed_threshold_kernel<<<(unsigned)ceil_div(n_query, 4), 128, 0, st>>>(
         w.seed, w.n_seed * 8, n_query, k_seed, w.q_resid, w.stats, w.gthr, sb ? std::max(1, sb->k_part) : 1,
@@ -1817,51 +1181,21 @@ int launch_sim_topk(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int t
     MCLST_CUDA(cudaMemsetAsync(w.spec, 0xff, (size_t)w.q_pad * sizeof(float), st));
   }
   if (phase == 1) return 0;
-#ifdef MCLST_TUNING_KNOBS
-  if (w.ring) {
-    auto launch_ring = [&](auto kern) -> int {
-      MCLST_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, RG_SMEM));
-      kern<<<grid, RG_THREADS, RG_SMEM, st>>>(p);
-      MCLST_LAUNCH_CHECK();
-      return 0;
-    };
-    if (w.cap == 256) return launch_ring(sim_topk_ring_kernel<256>);
-    if (w.cap == 512) return launch_ring(sim_topk_ring_kernel<512>);
-  }
-#endif
-  if (w.lanes && dump == nullptr) {
-    const LanePlan L = plan_lanes(w.q_pad / 128, p.tiles_total, sm_count(), std::max(1, 8 / (w.epw / 4)));
-    MCLST_REQUIRE(L.slots == w.S, MCLST_ERR_UNSUPPORTED, "sim_topk: lane plan changed (%d vs %d slots)", L.slots, w.S);
-    // slots a query block does not use must read as empty
-    MCLST_CUDA(cudaMemsetAsync(w.cand_cnt, 0, (size_t)w.q_pad * w.SS * sizeof(int), st));
-    auto launch_lanes = [&](auto kern, int threads) -> int {
-      // (all instantiations share one function-pointer type, hence one lambda body: no static flag)
-      MCLST_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM));
-      kern<<<(unsigned)L.W, threads, ST_SMEM, st>>>(p, L);
-      MCLST_LAUNCH_CHECK();
-      return 0;
-    };
-    if (w.cap == 256 && w.epw == 8) return launch_lanes(sim_topk_lanes_kernel<256, 8, false>, 64 + 32 * 8);
-    if (w.cap == 1024 && w.epw == 8) return launch_lanes(sim_topk_lanes_kernel<1024, 8, false>, 64 + 32 * 8);
-#ifdef MCLST_TUNING_KNOBS
-    if (w.cap == 256 && w.epw == 4) return launch_lanes(sim_topk_lanes_kernel<256, 4, false>, 64 + 32 * 4);
-    if (w.cap == 256 && w.epw == 16) return launch_lanes(sim_topk_lanes_kernel<256, 16, false>, 64 + 32 * 16);
-    if (w.cap == 1024 && w.epw == 4) return launch_lanes(sim_topk_lanes_kernel<1024, 4, false>, 64 + 32 * 4);
-#endif
-  }
-  // the (query block x stream) grid kernel: the debug similarity dump, and the lane kernel's
-  // predecessor in tuning builds
-  if (w.cap == 256) {
-    if (w.cluster == 1) return launch_sim_topk_e<256, 1>(w.epw, p, grid, st);
-#ifdef MCLST_TUNING_KNOBS
-    if (w.cluster == 2) return launch_sim_topk_e<256, 2>(w.epw, p, grid, st);
-    if (w.cluster == 4) return launch_sim_topk_e<256, 4>(w.epw, p, grid, st);
-#endif
-  } else if (w.cap == 1024) {
-    // large-k configurations (reference k = 200 / 600) are small problems: one variant
-    if (w.cluster == 1) return launch_sim_topk_e<1024, 1>(w.epw, p, grid, st);
-  }
-  MCLST_REQUIRE(false, MCLST_ERR_UNSUPPORTED, "sim_topk: cap %d cluster %d", w.cap, w.cluster);
+  // slots a query block does not use must read as empty
+  MCLST_CUDA(cudaMemsetAsync(w.cand_cnt, 0, (size_t)w.q_pad * w.SS * sizeof(int), st));
+  if (w.cap == 256) return launch_lanes<256, SimPass::Candidates>(p, w.plan, st);
+  // large-k configurations (reference k = 200 / 600) are small problems: one variant
+  if (w.cap == 1024) return launch_lanes<1024, SimPass::Candidates>(p, w.plan, st);
+  MCLST_REQUIRE(false, MCLST_ERR_UNSUPPORTED, "sim_topk: cap %d", w.cap);
+}
+
+int launch_sim_dump(const TcWorkspace& w, int64_t n_bank, int64_t n_query, float* dump, int64_t dump_ld,
+                    cudaStream_t st) {
+  SimParams p = sim_params(w, n_bank, n_query, 1);
+  p.dump = dump; p.dump_ld = dump_ld;
+  // the epilogue reads the shared thresholds whatever the pass: keep them defined
+  MCLST_CUDA(cudaMemsetAsync(w.gthr, 0, (size_t)w.q_pad * sizeof(uint32_t), st));
+  return launch_lanes<256, SimPass::Dump>(p, w.plan, st);
 }
 
 int launch_apply_bound(const TcWorkspace& w, int64_t n_query, const float* ext_bound, cudaStream_t st) {

@@ -1,5 +1,5 @@
-"""Per-kernel times of find_matches (+ distances) for one (N, Q) shape under the current
-MCLST_SIM_* environment.  usage: sim_sweep.py N Q [k]"""
+"""Per-kernel times of find_matches (+ distances) for one (N, Q) shape, averaged over 5 calls
+after 3 warm-ups.  usage: sim_sweep.py N Q [k]"""
 import sys, torch
 sys.path.insert(0, ".")
 from mclstexp_b200 import _lib, retrieval, synth
