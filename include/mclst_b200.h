@@ -183,6 +183,13 @@ int mclst_debug_spec_rank(int top_k, double sampled_fraction);
 int mclst_debug_lane_plan(int64_t query_blocks, int64_t bank_tiles, int lanes, int max_slots,
                           int* units, int64_t max_units, int64_t* n_units, int* slots);
 
+/* Testing aid (host only, no device needed): the tile kernel mclst_matmul's packed fp16 route runs
+ * for an M x N output with `batch` products, on the current device's SM count (148 without a
+ * device): *cluster = 2 for CTA pairs that share B (128 x 256 tiles) or 1, *width = the tile width
+ * 256, 128 or 64.  Honours MCLST_GEMM_CLUSTER like the launch does.  Not part of the reference
+ * surface. */
+int mclst_debug_gemm_variant(int64_t M, int64_t N, int batch, int* cluster, int* width);
+
 /* The whole fold-loop body (evel_her2st.py:174-187: find_matches, then the per-query loop) in ONE
  * call on device-resident arrays: out_indices [n_query, top_k] int64, out_values (nullable unless
  * MCLST_W_SIMILARITY) [n_query, top_k] float32, out_emb (nullable) [n_query, dim], out_expr

@@ -99,6 +99,7 @@ def load() -> C.CDLL:
     f64 = C.c_double
     lib.mclst_debug_spec_rank.argtypes = [i32, f64]
     lib.mclst_debug_lane_plan.argtypes = [i64, i64, i32, i32, p, i64, C.POINTER(i64), C.POINTER(i32)]
+    lib.mclst_debug_gemm_variant.argtypes = [i64, i64, i32, C.POINTER(i32), C.POINTER(i32)]
     lib.mclst_adam_coef_bytes.argtypes = [i32]
     lib.mclst_adam_coef_bytes.restype = sz
     lib.mclst_adam_set_step.argtypes = [p, i32, i32, f64, f64, f64, f64, f64, p]

@@ -788,6 +788,23 @@ static int launch_gemm_cl(const GemmParams& q, cudaStream_t st) {
   return 0;
 }
 
+// Which gemm_tn instantiation a product with an M x N x batch output runs on: *cluster = 2 (CTA pairs
+// sharing B, 128 x 256 tiles) or 1, *width = the tile width 256, 128 or 64.  narrow_ok is false for
+// products that need 256-wide tiles (fused row statistics, A concatenated along K).
+// MCLST_GEMM_CLUSTER=2 forces pairs, any other non-zero value forbids them.
+void gemm_variant(int64_t M, int64_t N, int batch, bool narrow_ok, int* cluster, int* width) {
+  static const int force = [] { const char* e = getenv("MCLST_GEMM_CLUSTER"); return e ? atoi(e) : 0; }();
+  const int64_t sms = sm_count();
+  const int64_t tiles = ceil_div(M, GM_BM) * ceil_div(N, GM_BN) * batch;
+  // pairs pay off once the grid is saturated and there are at least two row tiles to pair
+  const bool pair = force == 2 || (force == 0 && M > GM_BM && tiles >= 2 * sms);
+  *cluster = pair ? 2 : 1;
+  *width = 256;
+  // under-filled grid: half-width tiles, quarter-width once even those leave half of the SMs idle
+  if (!pair && narrow_ok && tiles < sms)
+    *width = 2 * ceil_div(M, GM_BM) * ceil_div(N, 128) * batch <= sms ? 64 : 128;
+}
+
 int launch_gemm_tn(const GemmParams& p, cudaStream_t st) {
   MCLST_REQUIRE(p.M > 0 && p.N > 0 && p.nkb > 0 && (p.nseg == 1 || p.nseg == 3), MCLST_ERR_INVALID,
                 "gemm: bad shape M=%lld N=%lld nkb=%d nseg=%d", (long long)p.M, (long long)p.N, p.nkb, p.nseg);
@@ -802,16 +819,13 @@ int launch_gemm_tn(const GemmParams& p, cudaStream_t st) {
   GemmParams q = p;
   q.batch = std::max(1, p.batch);
   prof_mark(st, "gemm_tn");
-  static const int force = [] { const char* e = getenv("MCLST_GEMM_CLUSTER"); return e ? atoi(e) : 0; }();
-  const int64_t tiles = ceil_div(p.M, GM_BM) * ceil_div(p.N, GM_BN) * q.batch;
-  // pairs pay off once the grid is saturated and there are at least two row tiles to pair
-  const bool pair = force == 2 || (force == 0 && p.M > GM_BM && tiles >= 2 * (int64_t)sm_count());
-  if (pair) return launch_gemm_cl<2, 256>(q, st);
-  // under-filled grid: half-width tiles (the fused row statistics are laid out for 256-wide tiles)
-  const bool narrow = !p.lse_part && p.a_nkb1 == 0 && tiles < (int64_t)sm_count();
-  if (!narrow) return launch_gemm_cl<1, 256>(q, st);
-  const int64_t tiles128 = ceil_div(p.M, GM_BM) * ceil_div(p.N, 128) * q.batch;
-  return 2 * tiles128 <= (int64_t)sm_count() ? launch_gemm_cl<1, 64>(q, st) : launch_gemm_cl<1, 128>(q, st);
+  int cluster, width;
+  // (the fused row statistics are laid out for 256-wide tiles)
+  gemm_variant(p.M, p.N, q.batch, !p.lse_part && p.a_nkb1 == 0, &cluster, &width);
+  if (cluster == 2) return launch_gemm_cl<2, 256>(q, st);
+  if (width == 64) return launch_gemm_cl<1, 64>(q, st);
+  if (width == 128) return launch_gemm_cl<1, 128>(q, st);
+  return launch_gemm_cl<1, 256>(q, st);
 }
 
 // ---- operand bookkeeping --------------------------------------------------------------
@@ -852,6 +866,12 @@ extern "C" int mclst_matmul_workspace_bytes(int64_t M, int64_t N, int64_t K, int
   take_operand(a, M, K, false, true, batch, true);
   take_operand(a, N, K, true, true, batch, true);
   *bytes = align_up(a.off, 256);
+  return 0;
+}
+
+extern "C" int mclst_debug_gemm_variant(int64_t M, int64_t N, int batch, int* cluster, int* width) {
+  MCLST_REQUIRE(cluster && width && M > 0 && N > 0 && batch >= 1, MCLST_ERR_INVALID, "gemm_variant: bad args");
+  gemm_variant(M, N, batch, true, cluster, width);
   return 0;
 }
 

@@ -111,4 +111,30 @@ def assert_grad_close(got, want, rtol=1e-3, rel_floor=2e-2, abs_cap=1e-4, elem_r
         f"{name}: element-wise relative {float(rel.max()):.3e} over {int(big.sum())} entries"
 
 
+def gemm_variant(M, N, batch=1):
+    """(cluster, tile width) of the tile kernel mclst_matmul's packed route runs for an M x N x batch
+    output on this device (mclst_debug_gemm_variant): (2, 256), (1, 256), (1, 128) or (1, 64)."""
+    import ctypes
+    from mclstexp_b200 import _lib
+    cl, w = ctypes.c_int(), ctypes.c_int()
+    _lib.check(_lib.load().mclst_debug_gemm_variant(M, N, batch, ctypes.byref(cl), ctypes.byref(w)),
+               "gemm_variant")
+    return cl.value, w.value
+
+
+def matmul_route(call):
+    """Runs call() -- one ops.matmul -- under the library's kernel trace and returns the route it took:
+    "tf32" (the 3xTF32 kernel that splits inside the K loop) or "packed" (pack_split, then gemm_tn)."""
+    from mclstexp_b200 import _lib
+    _lib.profile_enable(True)
+    try:
+        out = call()
+        names = [n for n, _ in _lib.profile_collect()]
+    finally:
+        _lib.profile_enable(False)
+    route = {("gemm_tf32",): "tf32", ("pack_split", "gemm_tn"): "packed"}.get(tuple(names))
+    assert route is not None, names
+    return route, out
+
+
 from oracle.oracle import find_matches_spec_rows  # noqa: E402,F401  (bank-chunked spec for a few rows)

@@ -2,8 +2,10 @@
 every symbol include/mclst_b200.h declares.  No compute calls (no GPU here)."""
 import numpy as np
 import ctypes
+import json
 import os
 import subprocess
+import sys
 
 import pytest
 
@@ -116,3 +118,57 @@ def test_speculative_seed_rank_is_the_binomial_tail():
                 assert tail(j - 1) >= 1e-7 or j == k
     assert lib.mclst_debug_spec_rank(50, 0.6) == 50                      # sampling most of the bank: no speculation
     assert lib.mclst_debug_spec_rank(5, 0.03) == 5                       # tiny k: none either
+
+
+def _sm_count(lib):
+    """The SM count mclst_debug_gemm_variant decides on: the device's, 148 (B200) without one."""
+    n = ctypes.c_int(0)
+    lib.mclst_device_info(ctypes.byref(n), None, None)
+    return n.value or 148
+
+
+def test_gemm_variant_follows_the_tile_rule(lib):
+    """csrc/gemm.cu gemm_variant, the tile kernel of mclst_matmul's packed route: CTA pairs (128 x 256
+    tiles, B shared) once there are two row tiles and at least two 128 x 256 tiles per SM; one CTA at
+    256-wide tiles while there is at least one per SM; below that 128-wide tiles, and 64-wide ones
+    while two 128-wide tiles still fit per SM."""
+    from checkers import gemm_variant
+    if os.environ.get("MCLST_GEMM_CLUSTER"):
+        pytest.skip("MCLST_GEMM_CLUSTER overrides the rule")
+    sms = _sm_count(lib)
+    cdiv = lambda a, b: -(-a // b)
+    seen = set()
+    for M in (1, 64, 128, 129, 256, 300, 1000, 2100, 5000):
+        for N in (1, 100, 128, 129, 256, 257, 700, 1000, 4096, 10000):
+            for batch in (1, 2, 3, 5, 8, 17, 33, 100, 1000):
+                cl, width = gemm_variant(M, N, batch)
+                seen.add((cl, width))
+                tiles256 = cdiv(M, 128) * cdiv(N, 256) * batch
+                tiles128 = cdiv(M, 128) * cdiv(N, 128) * batch
+                case = (M, N, batch, sms, cl, width)
+                assert (cl == 2) == (M > 128 and tiles256 >= 2 * sms), case
+                assert cl == 1 or width == 256, case
+                assert (width < 256) == (cl == 1 and tiles256 < sms), case
+                assert width != 64 or 2 * tiles128 <= sms, case
+                assert width != 128 or 2 * tiles128 > sms, case
+    assert seen == {(2, 256), (1, 256), (1, 128), (1, 64)}, seen
+    # a lone tile, and a product that fills every SM twice over in one row tile: SM-independent cases
+    assert gemm_variant(1, 1, 1) == (1, 64)
+    assert gemm_variant(128, 256 * 4 * sms, 1) == (1, 256)
+    assert gemm_variant(256, 256 * sms, 1) == (2, 256)
+    assert lib.mclst_debug_gemm_variant(0, 1, 1, ctypes.byref(ctypes.c_int()), ctypes.byref(ctypes.c_int())) == -1
+
+
+@pytest.mark.parametrize("force,want", [("2", (2, 256)), ("1", (1, 256))])
+def test_gemm_variant_honours_cluster_override(lib, force, want):
+    """MCLST_GEMM_CLUSTER=2 pairs every product, even a single row tile (its partner is a ghost);
+    any other value keeps the single-CTA kernels.  Read once per process, so checked in a fresh one."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    code = ("import json, sys; sys.path.insert(0, 'tests'); from checkers import gemm_variant; "
+            "print(json.dumps([gemm_variant(100, 700, 1), gemm_variant(5000, 10000, 8), gemm_variant(1, 1, 1)]))")
+    env = dict(os.environ, MCLST_GEMM_CLUSTER=force)
+    r = subprocess.run([sys.executable, "-c", code], env=env, cwd=root, capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr
+    small, big, one = (tuple(v) for v in json.loads(r.stdout.strip().splitlines()[-1]))
+    assert big == want
+    assert small == one == (want if force == "2" else (1, 64))

@@ -3,9 +3,18 @@ import numpy as np
 import pytest
 import torch
 
+from checkers import matmul_route
 from mclstexp_b200 import ops
 
 pytestmark = pytest.mark.gpu
+ROUTES = ["tf32", "packed"]
+
+
+def misaligned(t):
+    """A copy of the row-major matrix t whose base and rows are not 16-byte aligned: keeps a product
+    off the 3xTF32 kernel, which loads plain operands 16 bytes at a time."""
+    v = torch.empty(t.shape[0], t.shape[1] + 1, device="cuda")[:, 1:]
+    return v.copy_(t)
 
 
 @pytest.mark.parametrize("M,N,K", [(128, 256, 64), (1, 1, 1), (37, 300, 171), (1024, 1536, 785),
@@ -24,14 +33,20 @@ def test_matmul_nt_precise(M, N, K):
 
 
 def test_matmul_nt_epilogue():
+    """Bias, GELU and residual on both routes: the aligned operands take the 3xTF32 kernel, a
+    misaligned copy of A the packed one."""
     g = torch.Generator().manual_seed(5)
     M, N, K = 200, 333, 96
     a, b = torch.randn(M, K, generator=g), torch.randn(N, K, generator=g) * 0.2
     bias, res = torch.randn(N, generator=g), torch.randn(M, N, generator=g)
     want = torch.nn.functional.gelu(0.5 * a.double() @ b.double().T + bias.double()) + res.double()
-    got = ops.matmul_nt(a.cuda(), b.cuda(), alpha=0.5, bias=bias.cuda(), act="gelu",
-                        residual=res.cuda()).cpu().double()
-    assert (got - want).abs().max().item() <= 5e-6 * want.abs().max().item()
+    for route in ROUTES:
+        a_dev = a.cuda() if route == "tf32" else misaligned(a.cuda())
+        taken, got = matmul_route(lambda: ops.matmul_nt(a_dev, b.cuda(), alpha=0.5, bias=bias.cuda(), act="gelu",
+                                                        residual=res.cuda()))
+        assert taken == route
+        got = got.cpu().double()
+        assert (got - want).abs().max().item() <= 5e-6 * want.abs().max().item(), route
 
 
 def test_matmul_nt_strided_views():
@@ -76,19 +91,23 @@ def test_matmul_batched_head_slices():
     assert (out.double() - want).abs().max().item() <= 3e-5 * want.abs().max().item()
 
 
+@pytest.mark.parametrize("route", ROUTES)
 @pytest.mark.parametrize("sa,sb", [(1e-5, 1.0), (1e-5, 1e-5), (1e4, 1e4), (1e-30, 1e20), (3e30, 1e-12)])
 @pytest.mark.parametrize("a_trans,b_trans", [(False, False), (True, True)])
-def test_matmul_operand_magnitudes(sa, sb, a_trans, b_trans):
+def test_matmul_operand_magnitudes(sa, sb, a_trans, b_trans, route):
     """fp16 hi/lo halves have a 5-bit exponent: operands are brought into range with exact
     power-of-two row factors (gemm.cu), so gradients of magnitude 1e-5 and activations of 1e4
-    keep fp32-level accuracy (VERDICT r1 weak 6)."""
+    keep fp32-level accuracy (VERDICT r1 weak 6).  The 3xTF32 kernel needs no factors (8-bit
+    exponent) and must hold the same accuracy; K % 4 != 0 sends the product to the packed route."""
     g = torch.Generator().manual_seed(21)
-    M, N, K = 130, 270, 200
+    M, N, K = 130, 270, 200 if route == "tf32" else 201
     a = (torch.randn((K, M) if a_trans else (M, K), generator=g) * sa).cuda()
     b = (torch.randn((K, N) if b_trans else (N, K), generator=g) * sb).cuda()
     opa, opb = (a.T if a_trans else a), (b.T if b_trans else b)
     want = opa.double() @ opb.double().T
-    got = ops.matmul(a, b, a_trans, b_trans).double()
+    taken, got = matmul_route(lambda: ops.matmul(a, b, a_trans, b_trans))
+    assert taken == route
+    got = got.double()
     assert torch.isfinite(got).all()
     assert (got - want).abs().max().item() <= 3e-5 * want.abs().max().item()
 
@@ -114,14 +133,18 @@ def test_matmul_rows_of_very_different_scale_and_outliers():
 
 
 def test_matmul_non_finite_inputs_propagate():
+    """On both routes: the aligned operands take the 3xTF32 kernel, a misaligned copy of A the packed one."""
     a = torch.randn(40, 64).cuda()
     b = torch.randn(50, 64).cuda()
     a[2, 3] = float("inf")
     b[4, 5] = float("nan")
-    got = ops.matmul_nt(a, b)
-    assert not torch.isfinite(got[2]).any()          # inf * finite sums: inf or NaN, never a finite lie
-    assert torch.isnan(got[:, 4]).all()
-    assert torch.isfinite(got[[0, 1, 3]][:, [0, 1, 2, 3]]).all()
+    for route in ROUTES:
+        a_op = a if route == "tf32" else misaligned(a)
+        taken, got = matmul_route(lambda: ops.matmul_nt(a_op, b))
+        assert taken == route
+        assert not torch.isfinite(got[2]).any(), route      # inf * finite sums: inf or NaN, never a finite lie
+        assert torch.isnan(got[:, 4]).all(), route
+        assert torch.isfinite(got[[0, 1, 3]][:, [0, 1, 2, 3]]).all(), route
 
 
 @pytest.mark.parametrize("a_trans,b_trans", [(False, False), (False, True), (True, False), (True, True)])
