@@ -11,13 +11,17 @@
 //     dS = dLg I / T + (dA + dA^T) S a          dI = dLg^T S / T + (dA + dA^T) I a
 // (targets stay in the graph exactly as in the reference: the dA terms are their gradient).
 //
-// Execution: rows are processed in blocks of R (all of B when it fits the workspace).  Per
-// block three tensor-core products give the rows P1 = Lg_i., P2 = Lg_.i (= (I_i S^T)/T) and
-// P3 = A_i. ; three sweeps turn them into (1) rl, cl, za, (2) wbar, cs, loss, (3) the
-// gradient factors, which are written straight into TilePack operands and contracted with
-// [I;S]^T / [S;I]^T by two more tensor-core products.  All products use the 3-term fp16 split
-// (gemm.cu), i.e. fp32-level accuracy: logits reach +-256 here (LayerNorm'd embeddings have
-// norm 16), so single-pass fp16/bf16 operands cannot meet the 1e-3 gradient tolerance.
+// Execution: rows are processed in blocks of R (all of B when it fits the workspace).  When one
+// block holds the whole batch, the lean pipeline below runs.  Otherwise (a rank's slice of a
+// row-sharded batch, or a batch beyond the scratch budget) each block's tensor-core products give
+// the rows P1 = Lg_i., P2 = Lg_.i (= (I_i S^T)/T) and P3 = A_i., with the row log-sum-exp
+// partials of each product out of its epilogue; they are merged into rl, cl, za.  A sweep gives
+// wbar, cs and the loss, and a third pass the gradient factors, which are written straight into
+// TilePack operands and contracted with [I;S]^T / [S;I]^T by two more tensor-core products.  With
+// more than one block, phases 2 and 3 recompute each block's products.  All products use the
+// 3-term fp16 split (gemm.cu), i.e. fp32-level accuracy: logits reach +-256 here (LayerNorm'd
+// embeddings have norm 16), so single-pass fp16/bf16 operands cannot meet the 1e-3 gradient
+// tolerance.
 #include <algorithm>
 #include "common.cuh"
 #include "gemm.cuh"
@@ -27,15 +31,6 @@ namespace mclst {
 
 constexpr int LS_THREADS = 256;
 
-__device__ __forceinline__ float block_max(float v, float* sh) {
-  v = warp_max(v);
-  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
-  __syncthreads();
-  float r = sh[0];
-  for (int w = 1; w < LS_THREADS / 32; ++w) r = fmaxf(r, sh[w]);
-  __syncthreads();
-  return r;
-}
 __device__ __forceinline__ float block_sum(float v, float* sh) {
   v = warp_sum(v);
   if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
@@ -44,41 +39,6 @@ __device__ __forceinline__ float block_sum(float v, float* sh) {
   for (int w = 0; w < LS_THREADS / 32; ++w) r += sh[w];
   __syncthreads();
   return r;
-}
-
-// lse[r] = log sum_j exp(P[r, j]) over j < ncols; optionally diag[r] = P[r, row0 + r].
-// The statistic is kept as a float pair hi + lo (|lo| <= ulp(hi)/2): logits reach +-256 here, where
-// one float32 ulp is 3e-5 -- rounding rl / cl / za to a single float puts that much SYSTEMATIC error
-// into every exponent of the row and costs the small gradient entries a digit (measured: 1.5e-3
-// element-wise vs 1e-4 with the pair).  Consumers form exp((x - hi) - lo).
-__global__ void __launch_bounds__(LS_THREADS)
-row_lse_kernel(const float* __restrict__ P, int64_t ld, int ncols, int64_t row0,
-               float* __restrict__ lse, float* __restrict__ lse_lo, float* __restrict__ diag) {
-  __shared__ float sh[LS_THREADS / 32];
-  const int64_t r = blockIdx.x;
-  const float* p = P + r * ld;
-  // one pass: running (max, sum) pairs per thread, 16-byte loads over the 4-aligned body
-  float m = -INFINITY, s = 0.f;
-  auto push = [&](float x) {
-    if (x > m) { s = s * expf(m - x) + 1.f; m = x; }
-    else s += expf(x - m);
-  };
-  const int n4 = ((ld & 3) == 0) ? (ncols >> 2) : 0;
-  for (int j = threadIdx.x; j < n4; j += LS_THREADS) {
-    const float4 v = __ldg(reinterpret_cast<const float4*>(p) + j);
-    push(v.x); push(v.y); push(v.z); push(v.w);
-  }
-  for (int j = n4 * 4 + threadIdx.x; j < ncols; j += LS_THREADS) push(p[j]);
-  const float mb = block_max(m, sh);
-  s = block_sum(m == -INFINITY ? 0.f : s * expf(m - mb), sh);
-  m = mb;
-  if (threadIdx.x == 0) {
-    const double L = (double)m + log((double)s);
-    const float hi = (float)L;
-    lse[row0 + r] = hi;
-    lse_lo[row0 + r] = (hi == hi && fabsf(hi) < INFINITY) ? (float)(L - (double)hi) : 0.f;
-    if (diag) diag[row0 + r] = p[row0 + r];
-  }
 }
 
 // soft targets, sweep 2: wbar_r = sum_j Pt_rj W_rj ; cs_r = sum_j exp(A_rj - za_j)  (A symmetric)
@@ -247,11 +207,15 @@ grad_factor_kernel(const GradParams p, int64_t rows_pad) {
 //   wbar / cs sweep (soft targets)
 //   gradient factors per PAIR of mirrored 64 x 64 tiles: Lg_rj and Lg_jr, A_rj = A_jr are in
 //   shared memory together, so each exponential is evaluated once and P3 is read over the upper
-//   triangle only; G1 (dLg), G2 (dLg^T) and the symmetric Gs are written once each (12 B/element
-//   instead of 16 + a third product).
+//   triangle only; G1 (dLg) and the symmetric Gs are written once each (8 B/element instead of
+//   16 + a third product), and dI reads G1 transposed (MN-major tcgen05 descriptors).
 
 // partial (max, sum exp) pairs [slot][ld] -> float-pair statistic per row.  Slot s covers columns
 // [s * slot_cols, ...): slots starting at or beyond ncols were never written and are skipped.
+// The statistic is kept as a float pair hi + lo (|lo| <= ulp(hi)/2): logits reach +-256 here, where
+// one float32 ulp is 3e-5 -- rounding rl / cl / za to a single float puts that much SYSTEMATIC error
+// into every exponent of the row and costs the small gradient entries a digit (measured: 1.5e-3
+// element-wise vs 1e-4 with the pair).  Consumers form exp((x - hi) - lo).
 struct MergeJob { const float2* part; int slots, slot_cols, ncols; int64_t ld; float *hi, *lo; int n; };
 struct MergeJobs { MergeJob j[3]; };
 
@@ -314,7 +278,7 @@ struct TileGradParams {
   int B, soft;
   const float *rl, *cl, *za, *wbar, *cs, *rl_lo, *cl_lo, *za_lo;
   float inv_t, a_scale;            // normalised so that the stored factors are O(1)
-  uint8_t *g1_hi, *g1_lo, *g2_hi, *g2_lo, *gs_hi, *gs_lo;   // TilePack images [rows_pad, B64], K = batch index
+  uint8_t *g1_hi, *g1_lo, *gs_hi, *gs_lo;   // TilePack images [rows_pad, B64], K = batch index
   int nkb;                         // B64 / 64
 };
 
@@ -329,7 +293,7 @@ grad_tiles_kernel(const TileGradParams p) {
   const int tr = blockIdx.y, tc = blockIdx.x;
   if (tc < tr) return;                                   // the pair (tr, tc) also serves (tc, tr)
   extern __shared__ float tg_smem[];
-  float* sA = tg_smem;                                   // P1[tr rows][tc cols]   -> later g_rj
+  float* sA = tg_smem;                                   // P1[tr rows][tc cols]
   float* sB = sA + TG * TG_LD;                           // P1[tc rows][tr cols]   -> later g_jr
   float* sC = sB + TG * TG_LD;                           // P3[tr rows][tc cols]   -> later h
   float* st_r = sC + TG * TG_LD;                         // [8][64] statistics of the tr indices
@@ -403,11 +367,6 @@ grad_tiles_kernel(const TileGradParams p) {
 #pragma unroll
       for (int i = 0; i < 8; ++i) v[i] = g_rj[half * 8 + i];
       store_split(p.g1_hi, p.g1_lo, off, v);
-      if (p.g2_hi) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) v[i] = g_jr[half * 8 + i];
-        store_split(p.g2_hi, p.g2_lo, off, v);
-      }
       if (p.soft) {
 #pragma unroll
         for (int i = 0; i < 8; ++i) v[i] = h[half * 8 + i];
@@ -416,11 +375,10 @@ grad_tiles_kernel(const TileGradParams p) {
     }
   }
   if (tc == tr) return;                                  // (block-uniform)
-  // ---- mirrored tile (tc, tr): transpose the three result tiles through shared memory
+  // ---- mirrored tile (tc, tr): transpose the two result tiles through shared memory
   __syncthreads();                                       // everyone has read sA / sB / sC
 #pragma unroll
   for (int u = 0; u < 16; ++u) {
-    sA[r * TG_LD + jq + u] = g_rj[u];
     sB[r * TG_LD + jq + u] = g_jr[u];
     sC[r * TG_LD + jq + u] = h[u];
   }
@@ -436,11 +394,6 @@ grad_tiles_kernel(const TileGradParams p) {
 #pragma unroll
       for (int i = 0; i < 8; ++i) v[i] = sB[(rq + half * 8 + i) * TG_LD + j];      // dLg_jr as row j
       store_split(p.g1_hi, p.g1_lo, off, v);
-      if (p.g2_hi) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) v[i] = sA[(rq + half * 8 + i) * TG_LD + j];    // dLg_rj as its transpose
-        store_split(p.g2_hi, p.g2_lo, off, v);
-      }
       if (p.soft) {
 #pragma unroll
         for (int i = 0; i < 8; ++i) v[i] = sC[(rq + half * 8 + i) * TG_LD + j];
@@ -462,40 +415,25 @@ struct LossPlan {
   float *rl, *cl, *za, *wbar, *cs, *diag, *rl_lo, *cl_lo, *za_lo;   // views into the stats block [9][B]
   float* stats_ws;
   size_t bytes;
-  // lean single-block path
-  bool lean;
-  PackedOperand G1, G2, Gs;        // [R, B64] each
-  float2 *part1, *part2, *part3, *partc;   // LSE partials: rows of P1 / P2 / P3 [2 * nt256][R], columns of P1 [chunks][B64]
+  bool lean;                       // one row block holds the whole batch
+  PackedOperand G1, Gs;            // lean: [R, B64] each
+  // LSE partials: rows of P1 / P2 / P3 [2 * nt256][R] (P2 general, partc lean), columns of P1 [chunks][B64]
+  float2 *part1, *part2, *part3, *partc;
   int nt256, cchunks;
 };
 
-// MCLST_LOSS_LEAN=0 forces the general (row-blocked / row-sharded) pipeline on a whole batch too:
-// the tests use it to compare the two
-static bool lean_enabled() {
-  const char* e = getenv("MCLST_LOSS_LEAN");
-  return !(e && e[0] == '0');
-}
-// dI = dLg^T S + Gs I reads the dLg image TRANSPOSED (MN-major tcgen05 descriptors) instead of a
-// second, transposed copy of it: 4 of the 12 bytes per element the factor kernel writes.
-// MCLST_LOSS_MN=0 keeps the explicit copy (the tests compare the two).
-static bool mn_enabled() {
-  const char* e = getenv("MCLST_LOSS_MN");
-  return !(e && e[0] == '0');
-}
-
-static LossPlan plan_loss(void* ws, size_t cap, int B, int D, int soft, int want_grad, size_t budget,
-                          int64_t rows_local) {
+static LossPlan plan_loss(void* ws, size_t cap, int B, int D, int soft, size_t budget, int64_t rows_local) {
   LossPlan L{};
   L.B = B; L.D = D; L.soft = soft;
   L.B64 = (int64_t)align_up((size_t)B, 64);
   // row-block size: P1,P2,P3 (12 B/elem) + GA,GB hi/lo (8 or 16 B/elem) per (row, column)
-  const size_t per_row = (size_t)L.B64 * (12 + (want_grad ? (soft ? 16 : 8) : 0));
+  const size_t per_row = (size_t)L.B64 * (12 + (soft ? 16 : 8));
   int64_t R = (int64_t)(budget / std::max<size_t>(per_row, 1));
   R = std::max<int64_t>(128, R / 128 * 128);
   R = std::min<int64_t>(R, (int64_t)align_up((size_t)rows_local, 128));
   L.R = R;
   L.nblocks = ceil_div(rows_local, R);
-  L.lean = L.nblocks == 1 && rows_local == B && lean_enabled();
+  L.lean = L.nblocks == 1 && rows_local == B;
   L.nt256 = (int)ceil_div(B, 256);
   L.cchunks = (int)ceil_div(B, col_chunk_rows(B));
   Arena a(ws, cap);
@@ -504,27 +442,22 @@ static LossPlan plan_loss(void* ws, size_t cap, int B, int D, int soft, int want
   L.Ip = take_operand(a, B, D, true, true, 1);
   if (soft) L.ISp = take_operand(a, B, 2 * (int64_t)align_up((size_t)D, 64), true, true, 1);
   const int64_t kx = (soft ? 2 : 1) * L.B64;
-  if (want_grad) {
-    L.XT_IS = take_operand(a, D, kx, true, true, 1);
-    L.XT_SI = take_operand(a, D, kx, true, true, 1);
-    if (L.lean) {
-      L.G1 = take_operand(a, R, L.B64, false, true, 1);
-      if (!mn_enabled()) L.G2 = take_operand(a, R, L.B64, false, true, 1);
-      if (soft) L.Gs = take_operand(a, R, L.B64, false, true, 1);
-    } else {
-      L.GA = take_operand(a, R, kx, false, true, 1);
-      L.GB = take_operand(a, R, kx, false, true, 1);
-    }
+  L.XT_IS = take_operand(a, D, kx, true, true, 1);
+  L.XT_SI = take_operand(a, D, kx, true, true, 1);
+  if (L.lean) {
+    L.G1 = take_operand(a, R, L.B64, false, true, 1);
+    if (soft) L.Gs = take_operand(a, R, L.B64, false, true, 1);
+  } else {
+    L.GA = take_operand(a, R, kx, false, true, 1);
+    L.GB = take_operand(a, R, kx, false, true, 1);
   }
   L.P1 = a.take<float>((size_t)R * L.B64);
   L.P2 = L.lean ? nullptr : a.take<float>((size_t)R * L.B64);
   L.P3 = soft ? a.take<float>((size_t)R * L.B64) : nullptr;
-  if (L.lean || L.nblocks == 1) {
-    L.part1 = a.take<float2>((size_t)2 * L.nt256 * R);
-    L.part3 = soft ? a.take<float2>((size_t)2 * L.nt256 * R) : nullptr;
-    if (L.lean) L.partc = a.take<float2>((size_t)L.cchunks * L.B64);
-    else L.part2 = a.take<float2>((size_t)2 * L.nt256 * R);
-  }
+  L.part1 = a.take<float2>((size_t)2 * L.nt256 * R);
+  L.part3 = soft ? a.take<float2>((size_t)2 * L.nt256 * R) : nullptr;
+  if (L.lean) L.partc = a.take<float2>((size_t)L.cchunks * L.B64);
+  else L.part2 = a.take<float2>((size_t)2 * L.nt256 * R);
   L.stats_ws = a.take<float>((size_t)MCLST_LOSS_STAT_ROWS * B);
   L.bytes = align_up(a.off, 256);
   return L;
@@ -538,11 +471,13 @@ static size_t loss_budget() {
   return (size_t)(e ? atoll(e) : 32768) << 20;
 }
 
-// rows [i0, i0+rows) of P1 = S I^T / T, P2 = I S^T / T, P3 = [I|S][I|S]^T * a
-// with_stats: the row log-sum-exp partials (and the diagonal of P1) come out of the product
-// epilogues (part1 / part2 / part3, rows indexed locally) instead of three sweeps over the products
+// rows [i0, i0+rows) of P1 = S I^T / T, P2 = I S^T / T (need_p2), P3 = [I|S][I|S]^T * a, each with
+// its row log-sum-exp partials (part1 / part2 / part3, rows indexed locally) and P1 with its diagonal
+// out of the product epilogue.  The fused statistics fix the tile shape (gemm_variant), so a block
+// that phases 2 and 3 recompute is bit-identical to the one phase 1 took rl, cl, za from: the
+// softmax weights exp(A - za) of the recomputed rows then sum to one as exactly as in phase 1.
 static int compute_blocks(const LossPlan& L, int64_t i0, int64_t rows, float inv_t, float a_scale,
-                          bool need_p2, cudaStream_t st, bool with_stats = false) {
+                          bool need_p2, cudaStream_t st) {
   const int nkbD = L.Sp.nkb;
   GemmParams g{};
   g.nseg = 3; g.batch = 1; g.M = rows; g.N = L.B; g.ldc = L.B64;
@@ -552,30 +487,21 @@ static int compute_blocks(const LossPlan& L, int64_t i0, int64_t rows, float inv
   g.nkb = nkbD;
   g.a_hi = L.Sp.hi + a_off; g.a_lo = L.Sp.lo + a_off; g.b_hi = L.Ip.hi; g.b_lo = L.Ip.lo;
   g.c = L.P1; g.alpha = inv_t;
-  if (with_stats) { g.lse_part = L.part1; g.lse_ld = L.R; g.diag = L.diag + i0; g.diag_offset = i0; }
+  g.lse_part = L.part1; g.lse_ld = L.R; g.diag = L.diag + i0; g.diag_offset = i0;
   if ((rc = launch_gemm_tn(g, st))) return rc;
   g.diag = nullptr;
-  // small batches: one product is a handful of tiles (B = 1024: 32 of 148 SMs), and the products are
-  // independent -- the last one goes on the side stream, next to the first
-  const bool side_ok = L.soft && !need_p2 && ceil_div(rows, 128) * ceil_div(L.B, 256) * 2 <= sm_count();
-  cudaStream_t s3 = st;
-  if (side_ok && (rc = side_fork(st, &s3))) return rc;
   if (need_p2) {
     g.a_hi = L.Ip.hi + a_off; g.a_lo = L.Ip.lo + a_off; g.b_hi = L.Sp.hi; g.b_lo = L.Sp.lo;
-    g.c = L.P2;
-    if (with_stats) g.lse_part = L.part2;
+    g.c = L.P2; g.lse_part = L.part2;
     if ((rc = launch_gemm_tn(g, st))) return rc;
   }
   if (L.soft) {
     const size_t a2 = (size_t)(i0 / 128) * L.ISp.nkb * TP_SLICE_BYTES;
     g.nkb = L.ISp.nkb;
     g.a_hi = L.ISp.hi + a2; g.a_lo = L.ISp.lo + a2; g.b_hi = L.ISp.hi; g.b_lo = L.ISp.lo;
-    g.c = L.P3; g.alpha = a_scale;
-    if (with_stats) g.lse_part = L.part3;
-    if ((rc = launch_gemm_tn(g, s3))) return rc;
-    if (side_ok) prof_mark(s3, "end");
+    g.c = L.P3; g.alpha = a_scale; g.lse_part = L.part3;
+    if ((rc = launch_gemm_tn(g, st))) return rc;
   }
-  if (side_ok && (rc = side_join(st))) return rc;
   return 0;
 }
 
@@ -596,11 +522,10 @@ static int loss_phase(const float* spot_emb, int64_t ld_s, const float* image_em
                       float* d_image, int64_t ld_di, void* workspace, size_t workspace_bytes,
                       cudaStream_t st) {
   const int soft = target_mode != MCLST_T_EYE;
-  const int want_grad = 1;     // the layout always reserves the gradient operands (phase 3 may need them)
   const float inv_t = 1.0f / temperature;
   const float a_scale = target_mode == MCLST_T_SOFT_DIV ? 0.5f / temperature
                       : target_mode == MCLST_T_SOFT_MUL ? 0.5f * temperature : 0.f;
-  LossPlan L = plan_loss(workspace, workspace_bytes, B, D, soft, want_grad, loss_budget(), rows);
+  LossPlan L = plan_loss(workspace, workspace_bytes, B, D, soft, loss_budget(), rows);
   MCLST_REQUIRE(L.bytes <= workspace_bytes, MCLST_ERR_WORKSPACE, "contrastive_loss: workspace %zu < %zu",
                 workspace_bytes, L.bytes);
   bind_stats(L, stats ? stats : L.stats_ws);
@@ -631,53 +556,26 @@ static int loss_phase(const float* spot_emb, int64_t ld_s, const float* image_em
         if ((rc = launch_pack_split(image_emb, B, D, ld_i, true, 1.f, L.XT_SI, nkbB, nkbB, L.flags, nullptr, st))) return rc;
       }
     }
-    if (L.lean) {
-      // products with the row statistics fused into their epilogues; no transposed product
-      GemmParams g{};
-      g.nseg = 3; g.batch = 1; g.M = B; g.N = B; g.ldc = L.B64; g.amax_bits = L.flags; g.amax_pow = 2;
-      g.nkb = nkbD; g.a_hi = L.Sp.hi; g.a_lo = L.Sp.lo; g.b_hi = L.Ip.hi; g.b_lo = L.Ip.lo;
-      g.c = L.P1; g.alpha = inv_t; g.lse_part = L.part1; g.lse_ld = L.R; g.diag = L.diag; g.diag_offset = 0;
-      if ((rc = launch_gemm_tn(g, st))) return rc;
-      if (soft) {
-        g.nkb = L.ISp.nkb; g.a_hi = L.ISp.hi; g.a_lo = L.ISp.lo; g.b_hi = L.ISp.hi; g.b_lo = L.ISp.lo;
-        g.c = L.P3; g.alpha = a_scale; g.lse_part = L.part3; g.diag = nullptr;
-        if ((rc = launch_gemm_tn(g, st))) return rc;
-      }
-      prof_mark(st, "col_lse");
-      col_lse_partial_kernel<<<dim3((unsigned)ceil_div(B, 128), (unsigned)L.cchunks), 128, 0, st>>>(
-          L.P1, L.B64, B, B, col_chunk_rows(B), L.partc);
-      MCLST_LAUNCH_CHECK();
-      prof_mark(st, "lse_merge");
-      MergeJobs mj{};
-      mj.j[0] = MergeJob{L.part1, 2 * L.nt256, 128, B, L.R, L.rl, L.rl_lo, B};
-      mj.j[1] = MergeJob{L.partc, L.cchunks, 1, L.cchunks, L.B64, L.cl, L.cl_lo, B};
-      if (soft) mj.j[2] = MergeJob{L.part3, 2 * L.nt256, 128, B, L.R, L.za, L.za_lo, B};
-      lse_merge_kernel<<<dim3((unsigned)ceil_div(B, 256), soft ? 3u : 2u), 256, 0, st>>>(mj);
-      MCLST_LAUNCH_CHECK();
-    } else if (L.nblocks == 1) {
-      // one block holds this call's rows (a rank's slice of a sharded batch): statistics out of the
-      // product epilogues, the transposed product P2 supplies the column statistics of the local rows
-      if ((rc = compute_blocks(L, row0, rows, inv_t, a_scale, true, st, true))) return rc;
-      prof_mark(st, "lse_merge");
-      MergeJobs mj{};
-      mj.j[0] = MergeJob{L.part1, 2 * L.nt256, 128, B, L.R, L.rl + row0, L.rl_lo + row0, (int)rows};
-      mj.j[1] = MergeJob{L.part2, 2 * L.nt256, 128, B, L.R, L.cl + row0, L.cl_lo + row0, (int)rows};
-      if (soft) mj.j[2] = MergeJob{L.part3, 2 * L.nt256, 128, B, L.R, L.za + row0, L.za_lo + row0, (int)rows};
-      lse_merge_kernel<<<dim3((unsigned)ceil_div(rows, 256), soft ? 3u : 2u), 256, 0, st>>>(mj);
-      MCLST_LAUNCH_CHECK();
-    } else
+    // products with the row statistics fused into their epilogues, then one merge per row block.
+    // Lean: no transposed product; the column statistics come from a sweep over P1 instead.
     for (int64_t b = 0; b < L.nblocks; ++b) {
       const int64_t i0 = row0 + b * L.R, nr = std::min<int64_t>(L.R, row0 + rows - i0);
-      if ((rc = compute_blocks(L, i0, nr, inv_t, a_scale, true, st))) return rc;
-      prof_mark(st, "row_lse");
-      row_lse_kernel<<<(unsigned)nr, LS_THREADS, 0, st>>>(L.P1, L.B64, B, i0, L.rl, L.rl_lo, L.diag);
-      MCLST_LAUNCH_CHECK();
-      row_lse_kernel<<<(unsigned)nr, LS_THREADS, 0, st>>>(L.P2, L.B64, B, i0, L.cl, L.cl_lo, nullptr);
-      MCLST_LAUNCH_CHECK();
-      if (soft) {
-        row_lse_kernel<<<(unsigned)nr, LS_THREADS, 0, st>>>(L.P3, L.B64, B, i0, L.za, L.za_lo, nullptr);
+      if ((rc = compute_blocks(L, i0, nr, inv_t, a_scale, !L.lean, st))) return rc;
+      MergeJobs mj{};
+      mj.j[0] = MergeJob{L.part1, 2 * L.nt256, 128, B, L.R, L.rl + i0, L.rl_lo + i0, (int)nr};
+      if (L.lean) {
+        prof_mark(st, "col_lse");
+        col_lse_partial_kernel<<<dim3((unsigned)ceil_div(B, 128), (unsigned)L.cchunks), 128, 0, st>>>(
+            L.P1, L.B64, B, B, col_chunk_rows(B), L.partc);
         MCLST_LAUNCH_CHECK();
+        mj.j[1] = MergeJob{L.partc, L.cchunks, 1, L.cchunks, L.B64, L.cl, L.cl_lo, B};
+      } else {
+        mj.j[1] = MergeJob{L.part2, 2 * L.nt256, 128, B, L.R, L.cl + i0, L.cl_lo + i0, (int)nr};
       }
+      if (soft) mj.j[2] = MergeJob{L.part3, 2 * L.nt256, 128, B, L.R, L.za + i0, L.za_lo + i0, (int)nr};
+      prof_mark(st, "lse_merge");
+      lse_merge_kernel<<<dim3((unsigned)ceil_div(nr, 256), soft ? 3u : 2u), 256, 0, st>>>(mj);
+      MCLST_LAUNCH_CHECK();
     }
   } else if (phase == 2) {
     if (soft) {
@@ -702,7 +600,7 @@ static int loss_phase(const float* spot_emb, int64_t ld_s, const float* image_em
       tp.rl = L.rl; tp.cl = L.cl; tp.za = L.za; tp.wbar = L.wbar; tp.cs = L.cs;
       tp.rl_lo = L.rl_lo; tp.cl_lo = L.cl_lo; tp.za_lo = L.za_lo;
       tp.inv_t = inv_t / u; tp.a_scale = a_scale / u;
-      tp.g1_hi = L.G1.hi; tp.g1_lo = L.G1.lo; tp.g2_hi = L.G2.hi; tp.g2_lo = L.G2.lo;
+      tp.g1_hi = L.G1.hi; tp.g1_lo = L.G1.lo;
       tp.gs_hi = L.Gs.hi; tp.gs_lo = L.Gs.lo; tp.nkb = L.G1.nkb;
       static bool attr_set = false;
       if (!attr_set) {
@@ -726,12 +624,10 @@ static int loss_phase(const float* spot_emb, int64_t ld_s, const float* image_em
       cudaStream_t s2 = st;
       if (pair && (rc = side_fork(st, &s2))) return rc;
       if ((rc = launch_gemm_tn(g, st))) return rc;
-      if (L.G2.hi) {
-        g.a_hi = L.G2.hi; g.a_lo = L.G2.lo;
-      } else {                               // dLg^T: the same image, read MN-major
-        g.a1_mn = L.G1.nkb;
-        g.a_nkb1 = L.G1.nkb;                 // (eye targets: image 1 is the whole K range)
-      }
+      // dI = dLg^T S + Gs I reads the dLg image TRANSPOSED (MN-major tcgen05 descriptors) instead of
+      // a second, transposed copy of it (4 more bytes per element for the factor kernel to write)
+      g.a1_mn = L.G1.nkb;
+      g.a_nkb1 = L.G1.nkb;                   // (eye targets: image 1 is the whole K range)
       g.b_hi = L.XT_SI.hi; g.b_lo = L.XT_SI.lo;
       g.c = d_image; g.ldc = ld_di;
       if ((rc = launch_gemm_tn(g, s2))) return rc;
@@ -781,7 +677,7 @@ extern "C" int mclst_contrastive_loss_workspace_bytes(int batch, int dim, int ta
   MCLST_REQUIRE(bytes && batch >= 1 && dim >= 1 && target_mode >= 0 && target_mode <= 2 &&
                 rows_local >= 1 && rows_local <= batch, MCLST_ERR_INVALID,
                 "contrastive_loss_workspace: bad args");
-  *bytes = plan_loss(nullptr, 0, batch, dim, target_mode != MCLST_T_EYE, 1, loss_budget(), rows_local).bytes;
+  *bytes = plan_loss(nullptr, 0, batch, dim, target_mode != MCLST_T_EYE, loss_budget(), rows_local).bytes;
   return 0;
 }
 
