@@ -87,7 +87,10 @@ int mclst_profile_collect(char* names_out, float* ms_out, int cap, int* n);
  * cosine similarity per query and return the top_k, sorted by (similarity descending,
  * index ascending).  out_indices [n_query, top_k] int64 (torch.topk's dtype), each index
  * + index_offset (bank shards).  out_values (nullable) [n_query, top_k] float32 are the
- * similarities the cSCC flavour returns. */
+ * similarities the cSCC flavour returns.  Any dim works; the output is always the exact one.
+ * Calls with dim <= 512, top_k <= 896 and top_k <= n_bank (mclst_find_matches_tc_eligible) run
+ * the tensor-core candidate pass plus an exact re-rank; all others, and MCLST_FM_EXACT_ONLY,
+ * brute-force every query in float64. */
 int mclst_find_matches_workspace_bytes(int64_t n_bank, int64_t n_query, int dim, int top_k,
                                        int flags, size_t* bytes);
 int mclst_find_matches(const float* bank, int64_t n_bank, int64_t ld_bank,
@@ -162,9 +165,14 @@ int mclst_find_matches_finish(const float* bank, int64_t n_bank, int64_t ld_bank
                               const float* ext_bound, void* workspace, size_t workspace_bytes,
                               int flags, mclst_stream_t stream);
 
+/* 1 if a find_matches call of this shape and flags runs the tensor-core candidate pass, 0 if it
+ * brute-forces every query: !(flags & MCLST_FM_EXACT_ONLY) && 1 <= dim <= 512 && top_k <= 896
+ * && top_k <= n_bank.  MCLST_FM_BANK_PACKED needs it.  Host only, no device needed. */
+int mclst_find_matches_tc_eligible(int64_t n_bank, int dim, int top_k, int flags);
+
 /* Testing aid: the raw similarities of the tensor-core candidate pass (fp16-rounded
- * normalised operands, fp32 accumulation) written to out [n_query, ld_out]; workspace as for
- * mclst_find_matches with top_k = 1.  Not part of the reference surface. */
+ * normalised operands, fp32 accumulation) written to out [n_query, ld_out]; dim <= 512;
+ * workspace as for mclst_find_matches with top_k = 1.  Not part of the reference surface. */
 int mclst_debug_similarity(const float* bank, int64_t n_bank, int64_t ld_bank,
                            const float* query, int64_t n_query, int64_t ld_query, int dim,
                            float* out, int64_t ld_out, void* workspace, size_t workspace_bytes,

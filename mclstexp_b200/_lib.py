@@ -54,6 +54,7 @@ def load() -> C.CDLL:
     lib.mclst_profile_collect.argtypes = [C.c_char_p, C.POINTER(C.c_float), i32, C.POINTER(i32)]
     lib.mclst_read_counters.argtypes = [p, C.POINTER(i64), p]
     lib.mclst_find_matches_workspace_bytes.argtypes = [i64, i64, i32, i32, i32, C.POINTER(sz)]
+    lib.mclst_find_matches_tc_eligible.argtypes = [i64, i32, i32, i32]
     lib.mclst_find_matches.argtypes = [p, i64, i64, p, i64, i64, i32, i32, i64, p, p, p, sz, i32, p]
     lib.mclst_find_matches_pack_bank.argtypes = [p, i64, i64, i32, i32, p, sz, p]
     lib.mclst_find_matches_seed.argtypes = [p, i64, i64, p, i64, i64, i32, i32, i32, p, p, p, sz, i32, p]

@@ -65,9 +65,10 @@ struct FmWorkspace {
   size_t bytes;
 };
 
-static bool tc_eligible(int64_t n_bank, int64_t n_query, int dim, int top_k, int flags) {
-  (void)n_query;
-  return !(flags & MCLST_FM_EXACT_ONLY) && dim <= 256 && tc_cap_for_k(top_k) != 0 &&
+// The one eligibility rule of the tensor-core candidate path (exported as
+// mclst_find_matches_tc_eligible; the Python layers ask it instead of restating it).
+static bool tc_eligible(int64_t n_bank, int dim, int top_k, int flags) {
+  return !(flags & MCLST_FM_EXACT_ONLY) && dim >= 1 && dim <= TC_MAX_DIM && tc_cap_for_k(top_k) != 0 &&
          n_bank >= top_k;
 }
 
@@ -76,7 +77,7 @@ static FmWorkspace carve_fm(void* ws, size_t cap, int64_t n_bank, int64_t n_quer
   Arena a(ws, cap);
   FmWorkspace w{};
   w.counters = a.take<int>(64);
-  w.use_tc = tc_eligible(n_bank, n_query, dim, top_k, flags);
+  w.use_tc = tc_eligible(n_bank, dim, top_k, flags);
   if (w.use_tc) {
     tc_workspace(a, n_bank, n_query, dim, top_k, w.tc);
     w.tc.speculate = (flags & MCLST_FM_NO_SPECULATION) ? 0 : 1;
@@ -167,6 +168,10 @@ extern "C" int mclst_find_matches_workspace_bytes(int64_t n_bank, int64_t n_quer
   return 0;
 }
 
+extern "C" int mclst_find_matches_tc_eligible(int64_t n_bank, int dim, int top_k, int flags) {
+  return tc_eligible(n_bank, dim, top_k, flags) ? 1 : 0;
+}
+
 extern "C" int mclst_find_matches_dist(const float* bank, int64_t n_bank, int64_t ld_bank,
                                        const float* query, int64_t n_query, int64_t ld_query,
                                        int dim, int top_k, int64_t index_offset,
@@ -209,7 +214,8 @@ static int find_matches_stages(int stages, const float* bank, int64_t n_bank, in
                 "find_matches: workspace %zu < %zu", workspace_bytes, w.bytes);
   const bool packed = (flags & MCLST_FM_BANK_PACKED) != 0;
   MCLST_REQUIRE(!packed || w.use_tc, MCLST_ERR_INVALID,
-                "find_matches: MCLST_FM_BANK_PACKED needs the tensor-core path (dim <= 256, k <= 896)");
+                "find_matches: MCLST_FM_BANK_PACKED needs the tensor-core path (dim <= %d, k <= 896, k <= n_bank)",
+                TC_MAX_DIM);
   int rc;
   if (!w.use_tc) {
     if (stages & 1) {
@@ -481,7 +487,7 @@ extern "C" int mclst_retrieve(const float* bank, int64_t n_bank, int64_t ld_bank
     const int64_t nq = std::min(QB, n_query - q0);
     // the bank is packed by the first block; later blocks find its image at the head of the workspace
     const int f = flags | (b > 0 ? MCLST_FM_BANK_PACKED : 0);
-    const bool tc = tc_eligible(n_bank, nq, dim, top_k, f);
+    const bool tc = tc_eligible(n_bank, dim, top_k, f);
     rc = find_matches_stages(7, bank, n_bank, ld_bank, query + q0 * ld_query, nq, ld_query, dim, top_k, 0,
                              out_indices + q0 * top_k, out_values ? out_values + q0 * top_k : nullptr,
                              dist ? dist + q0 * top_k : nullptr, dist_p, nullptr, workspace, fm_bytes,
@@ -516,7 +522,8 @@ extern "C" int mclst_debug_similarity(const float* bank, int64_t n_bank, int64_t
                                       int dim, float* out, int64_t ld_out, void* workspace,
                                       size_t workspace_bytes, mclst_stream_t stream) {
   MCLST_REQUIRE(bank && query && out && workspace, MCLST_ERR_INVALID, "debug_similarity: null");
-  MCLST_REQUIRE(dim >= 1 && dim <= 256, MCLST_ERR_UNSUPPORTED, "debug_similarity: dim");
+  MCLST_REQUIRE(dim >= 1 && dim <= TC_MAX_DIM, MCLST_ERR_UNSUPPORTED, "debug_similarity: dim %d > %d", dim,
+                TC_MAX_DIM);
   cudaStream_t st = (cudaStream_t)stream;
   FmWorkspace w = carve_fm(workspace, workspace_bytes, n_bank, n_query, dim, 1, 0);
   MCLST_REQUIRE(w.use_tc && w.bytes <= workspace_bytes, MCLST_ERR_WORKSPACE, "debug_similarity: ws");

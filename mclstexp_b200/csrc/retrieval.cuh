@@ -17,6 +17,7 @@ int launch_exact_topk(const float* bank, int64_t N, int64_t ldb, const double* b
                       float* out_val, cudaStream_t st);
 
 // ---- tensor-core candidate path (sim_topk.cu)
+constexpr int TC_MAX_DIM = 512;   // widest rows it takes (the resident query block of the wide variant)
 // Work decomposition of the persistent candidate kernel: W lanes (CTAs) walk closed-form unit
 // lists (sim_topk.cu: plan_lanes / lane_unit); `slots` candidate slots per query block.
 struct LanePlan {
@@ -25,6 +26,7 @@ struct LanePlan {
 };
 struct TcWorkspace {
   int nkb, SS, cap;         // SS = 2 * plan.slots candidate streams per query (two column halves)
+  float e_acc;              // accumulation bound of this width (sim_topk.cu: E_ACC, E_ACC_WIDE)
   LanePlan plan;            // of the candidate pass
   int64_t q_pad, n_pad;
   uint32_t* stats;          // [0..7] bank: max residual bits, non-finite flag; [8..15] queries

@@ -4,8 +4,9 @@
 //   pack_rows      fp32 rows -> L2-normalised fp16 "TilePack" operand (+ norm, fp16 rounding
 //                  residual per row).  HBM-bound, one warp per row.
 //   sim_topk       persistent-per-CTA GEMM: 128 queries (TMEM lanes) x 256 bank rows (TMEM
-//                  columns) per tile, K = 256.  Warp 0 streams bank slices with cp.async.bulk
-//                  (TMA engine) into a 4-stage shared-memory ring, warp 1 issues
+//                  columns) per tile, K <= 512.  Warp 0 streams bank slices with cp.async.bulk
+//                  (TMA engine) into a 4-stage (K <= 256) or 3-stage (K <= 512) shared-memory
+//                  ring, warp 1 issues
 //                  tcgen05.mma.kind::f16 into a double-buffered 2 x 256-column TMEM
 //                  accumulator, warps 2-9 drain it with tcgen05.ld: every thread owns one
 //                  query row, compares 32 similarities per load against its running
@@ -19,7 +20,7 @@
 // Exactness argument (DESIGN.md "retrieval/exactness"): with |approx - exact| <= eps for
 // every (query, row) pair -- eps = (r_q + max_s r_s) * (1 + 2^-9) + E_ACC, r = fp16 rounding
 // residual norms measured at pack time (Cauchy-Schwarz), E_ACC the tensor-core accumulation
-// bound -- any row whose approximate score is below (k-th best approximate) - 2*eps is
+// bound (E_ACC_WIDE for K > 256) -- any row whose approximate score is below (k-th best approximate) - 2*eps is
 // strictly worse than k rows, so it cannot be in the exact top-k.  The running threshold
 // only ever uses a LOWER bound of the running k-th best, so nothing needed is dropped.
 // Rows for which the band overflows the candidate buffer (massive ties, pathological
@@ -36,13 +37,18 @@ using namespace ptx;
 // Bound on the tcgen05 fp32 accumulation error for |scores| <= 1, K <= 256.  Measured on
 // B200 (tests/test_simtopk_gpu.py): max 1.5e-7 -- the bound keeps a 13x margin.
 constexpr float E_ACC = 2.0e-6f;
+// The same for 256 < K <= 512 (twice the accumulation steps, twice the bound).  Measured on B200
+// (tests/test_retrieval_wide_gpu.py): max 2.3e-7 at K = 512 -- a 17x margin.  Each call carries
+// the bound of its width (TcWorkspace::e_acc), so the bands and candidate counts of K <= 256 do
+// not move.
+constexpr float E_ACC_WIDE = 4.0e-6f;
 
 // ============================================================================ pack_rows
-// One warp per row (grid-stride), dim <= 256: lane l owns elements 8l..8l+7 (one 16-byte fp16
-// chunk).  Per-row statistics are reduced per block before touching the global maximum: one
-// atomic per row on a single address made the first version L2-atomic bound (1.3 ms for 1.06 M
-// rows, 14 % of DRAM bandwidth).
-template <bool VEC>
+// One warp per row (grid-stride).  CPL = 16-byte fp16 chunks per lane: 1 for dim <= 256 (lane l
+// owns elements 8l..8l+7), 2 for dim <= 512 (chunks l and l + 32).  Per-row statistics are
+// reduced per block before touching the global maximum: one atomic per row on a single address
+// made the first version L2-atomic bound (1.3 ms for 1.06 M rows, 14 % of DRAM bandwidth).
+template <bool VEC, int CPL>
 __global__ void __launch_bounds__(256)
 pack_rows_kernel(const float* __restrict__ x, int64_t rows, int64_t rows_pad, int64_t ld, int dim,
                  int nkb, uint8_t* __restrict__ packed, double* __restrict__ nrm,
@@ -50,40 +56,44 @@ pack_rows_kernel(const float* __restrict__ x, int64_t rows, int64_t rows_pad, in
   __shared__ uint32_t s_max[8];
   __shared__ uint32_t s_bad[8];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int nchunks = nkb * 8;               // 16-byte chunks (8 halves) per row; <= 32
+  const int nchunks = nkb * 8;               // 16-byte chunks (8 halves) per row; <= 32 * CPL
   float run_max = 0.f;
   uint32_t run_bad = 0u;
   for (int64_t r = (int64_t)blockIdx.x * 8 + warp; r < rows_pad; r += (int64_t)gridDim.x * 8) {
-    float v[8];
+    float v[8 * CPL];
 #pragma unroll
-    for (int i = 0; i < 8; ++i) v[i] = 0.f;
-    if (r < rows && lane < nchunks) {
-      const float* p = x + r * ld + lane * 8;
-      if (VEC) {                               // dim % 8 == 0, 16-byte aligned rows
-        if (lane * 8 < dim) {
-          const float4 a = ldg_stream(reinterpret_cast<const float4*>(p));
-          const float4 b = ldg_stream(reinterpret_cast<const float4*>(p) + 1);
-          v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w;
-          v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+    for (int i = 0; i < 8 * CPL; ++i) v[i] = 0.f;
+#pragma unroll
+    for (int c = 0; c < CPL; ++c) {
+      const int chunk = lane + 32 * c;
+      if (r < rows && chunk < nchunks) {
+        const float* p = x + r * ld + chunk * 8;
+        if (VEC) {                               // dim % 8 == 0, 16-byte aligned rows
+          if (chunk * 8 < dim) {
+            const float4 a = ldg_stream(reinterpret_cast<const float4*>(p));
+            const float4 b = ldg_stream(reinterpret_cast<const float4*>(p) + 1);
+            v[8 * c + 0] = a.x; v[8 * c + 1] = a.y; v[8 * c + 2] = a.z; v[8 * c + 3] = a.w;
+            v[8 * c + 4] = b.x; v[8 * c + 5] = b.y; v[8 * c + 6] = b.z; v[8 * c + 7] = b.w;
+          }
+        } else {
+#pragma unroll
+          for (int i = 0; i < 8; ++i)
+            if (chunk * 8 + i < dim) v[8 * c + i] = __ldg(p + i);
         }
-      } else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i)
-          if (lane * 8 + i < dim) v[i] = __ldg(p + i);
       }
     }
     double ss = 0.0;
 #pragma unroll
-    for (int i = 0; i < 8; ++i) ss = fma((double)v[i], (double)v[i], ss);
+    for (int i = 0; i < 8 * CPL; ++i) ss = fma((double)v[i], (double)v[i], ss);
     ss = warp_sum(ss);
     const double n64 = fmax(sqrt(ss), 1e-12);
     // the fp16 operand only has to be an accurate normalisation (its rounding residual is
     // measured below and the 1e-6 slack of pair_eps covers the 2-ulp reciprocal)
     const float inv = (float)(1.0 / n64);
     float res = 0.f;
-    uint32_t h2[4];
+    uint32_t h2[4 * CPL];
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < 4 * CPL; ++i) {
       const float a = v[2 * i] * inv, b = v[2 * i + 1] * inv;
       const __half ha = __float2half_rn(a), hb = __float2half_rn(b);
       const float da = a - __half2float(ha), db = b - __half2float(hb);
@@ -92,9 +102,13 @@ pack_rows_kernel(const float* __restrict__ x, int64_t rows, int64_t rows_pad, in
       h2[i] = (uint32_t)__half_as_ushort(ha) | ((uint32_t)__half_as_ushort(hb) << 16);
     }
     res = warp_sum(res);
-    if (lane < nchunks)
-      *reinterpret_cast<uint4*>(packed + tilepack_chunk_offset(r, lane, nkb)) =
-          make_uint4(h2[0], h2[1], h2[2], h2[3]);
+#pragma unroll
+    for (int c = 0; c < CPL; ++c) {
+      const int chunk = lane + 32 * c;
+      if (chunk < nchunks)
+        *reinterpret_cast<uint4*>(packed + tilepack_chunk_offset(r, chunk, nkb)) =
+            make_uint4(h2[4 * c], h2[4 * c + 1], h2[4 * c + 2], h2[4 * c + 3]);
+    }
     if (lane == 0) {
       const float rr = (r < rows) ? sqrtf(res) * 1.00001f + 1e-12f : 0.f;
       nrm[r] = n64;
@@ -120,7 +134,16 @@ constexpr int ST_STAGES = 4;
 constexpr int ST_BN = 256;                      // bank rows per tile (TMEM columns)
 constexpr int ST_STAGE_BYTES = 2 * TP_SLICE_BYTES;   // 256 rows x 64 halves
 constexpr int ST_A_BYTES = 4 * TP_SLICE_BYTES;       // up to 4 K slices (dim <= 256)
-constexpr int ST_SMEM = ST_A_BYTES + ST_STAGES * ST_STAGE_BYTES + 1024 /*barriers*/ + 1024 /*align*/;
+// Wide variant (256 < dim <= 512): the resident query block takes 8 K slices (128 KiB), so the
+// bank ring drops to 3 stages: 128 + 3 x 32 + 2 KiB = 231 424 B fits the 232 448 B opt-in limit,
+// 4 stages would not.
+constexpr int ST_STAGES_WIDE = 3;
+constexpr int ST_A_BYTES_WIDE = 8 * TP_SLICE_BYTES;
+static_assert(ST_A_BYTES_WIDE == TC_MAX_DIM / TP_K * TP_SLICE_BYTES, "resident query block of the widest rows");
+constexpr int st_smem(int a_bytes, int stages) {
+  return a_bytes + stages * ST_STAGE_BYTES + 1024 /*barriers*/ + 1024 /*align*/;
+}
+static_assert(st_smem(ST_A_BYTES_WIDE, ST_STAGES_WIDE) <= 232448, "wide sim_topk exceeds the shared-memory opt-in limit");
 // Epilogue warps.  TMEM lanes can only be read by the warp whose id % 4 matches the lane quadrant,
 // so two warps share a quadrant and split the 256 columns of a tile between them; each (query,
 // column part) is its own candidate stream.  One epilogue warp per scheduler cannot hide its own
@@ -156,12 +179,14 @@ struct SimParams {
   // 32-score chunk into seed_out [q_pad][n_tiles * 8] (no candidates, no thresholds)
   float* seed_out;
   int tile_begin, tile_stride, n_tiles;
+  float e_acc;          // accumulation bound of this width (pair_eps); sits in the tail padding
 };
 
 // eps: |tensor-core score - exact cosine| for a pair with fp16 residual norms rq, rs
-// (Cauchy-Schwarz on the operand rounding) + accumulation bound + fp32 normalisation slack.
-__device__ __forceinline__ float pair_eps(float rq, float rs) {
-  return 1.002f * (rq + rs) + E_ACC + 1e-6f;
+// (Cauchy-Schwarz on the operand rounding) + accumulation bound e_acc of the call's width
+// (E_ACC or E_ACC_WIDE) + fp32 normalisation slack.
+__device__ __forceinline__ float pair_eps(float rq, float rs, float e_acc) {
+  return 1.002f * (rq + rs) + e_acc + 1e-6f;
 }
 
 // Warp-cooperative prune of the candidate buffers of every lane with need == true:
@@ -422,8 +447,10 @@ static LanePlan plan_lanes(int64_t qt, int64_t T, int W, int max_slots) {
 }
 
 // PASS (SimPass) selects what the epilogue does with the scores of a tile.  In the Seed pass
-// "tile" t of a unit is bank tile tile_begin + t * tile_stride of the sample.
-template <int CAP, SimPass PASS>
+// "tile" t of a unit is bank tile tile_begin + t * tile_stride of the sample.  A_BYTES (resident
+// query block) and STAGES (bank ring) are ST_A_BYTES / ST_STAGES for dim <= 256 and
+// ST_A_BYTES_WIDE / ST_STAGES_WIDE for dim <= 512; nothing else depends on the width.
+template <int CAP, SimPass PASS, int A_BYTES, int STAGES>
 __global__ void __launch_bounds__(ST_THREADS, 1)
 sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
   constexpr bool SEED = PASS == SimPass::Seed;
@@ -432,10 +459,10 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
   uint8_t* sA = smem;
-  uint8_t* sB = smem + ST_A_BYTES;
-  uint64_t* bar_full = reinterpret_cast<uint64_t*>(sB + ST_STAGES * ST_STAGE_BYTES);
-  uint64_t* bar_empty = bar_full + ST_STAGES;
-  uint64_t* bar_a = bar_empty + ST_STAGES;
+  uint8_t* sB = smem + A_BYTES;
+  uint64_t* bar_full = reinterpret_cast<uint64_t*>(sB + STAGES * ST_STAGE_BYTES);
+  uint64_t* bar_empty = bar_full + STAGES;
+  uint64_t* bar_a = bar_empty + STAGES;
   uint64_t* bar_afree = bar_a + 1;
   uint64_t* bar_tfull = bar_afree + 1;
   uint64_t* bar_tempty = bar_tfull + 2;
@@ -447,7 +474,7 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
   const int T = SEED ? p.n_tiles : p.tiles_total;
 
   if (threadIdx.x == 0) {
-    for (int i = 0; i < ST_STAGES; ++i) { mbar_init(&bar_full[i], 1); mbar_init(&bar_empty[i], 1); }
+    for (int i = 0; i < STAGES; ++i) { mbar_init(&bar_full[i], 1); mbar_init(&bar_empty[i], 1); }
     mbar_init(bar_a, 1);
     mbar_init(bar_afree, 1);
     for (int i = 0; i < 2; ++i) { mbar_init(&bar_tfull[i], 1); mbar_init(&bar_tempty[i], ST_EPW); }
@@ -483,7 +510,7 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
                           &bar_full[stage], pol_keep);
             bulk_g2s_hint(dst + TP_SLICE_BYTES, p.bpack + ((size_t)(2 * bt + 1) * nkb + kb) * TP_SLICE_BYTES,
                           TP_SLICE_BYTES, &bar_full[stage], pol_keep);
-            if (++stage == ST_STAGES) { stage = 0; phase ^= 1; }
+            if (++stage == STAGES) { stage = 0; phase ^= 1; }
           }
         }
       }
@@ -520,7 +547,7 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
             mma_commit(&bar_empty[stage]);
           }
           __syncwarp();
-          if (++stage == ST_STAGES) { stage = 0; phase ^= 1; }
+          if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
         if (leader) mma_commit(&bar_tfull[buf]);
         __syncwarp();
@@ -551,7 +578,7 @@ sim_topk_lanes_kernel(const SimParams p, const LanePlan L) {
       uint2* my_buf = p.cand + ((size_t)q * SS + stream) * CAP;
       uint32_t* my_gthr = p.gthr + q;
       const float rq = q_valid ? p.q_resid[q] : 0.f;
-      const float e2 = 2.02f * pair_eps(rq, rs_max);
+      const float e2 = 2.02f * pair_eps(rq, rs_max, p.e_acc);
       float thr = q_valid ? __int_as_float(0xff800000) : __int_as_float(0x7f800000);
       int cnt = 0;
       int flagged = 0;
@@ -629,7 +656,7 @@ __global__ void __launch_bounds__(128)
 seed_threshold_kernel(const float* __restrict__ seed, int n_vals, int64_t Q, int k,
                       const float* __restrict__ q_resid, const uint32_t* __restrict__ bank_stats,
                       uint32_t* __restrict__ gthr, int k2, float* __restrict__ bound_k,
-                      float* __restrict__ bound_part, float* __restrict__ spec_out) {
+                      float* __restrict__ bound_part, float* __restrict__ spec_out, float e_acc) {
   // k < top_k is the SPECULATIVE start (see spec_rank): the threshold is then only valid if fewer
   // than k of the true top rows fell into the sample; spec_out records it so that the re-rank can
   // verify the outcome with one compare (and send the query to the exact path otherwise).
@@ -680,7 +707,7 @@ seed_threshold_kernel(const float* __restrict__ seed, int n_vals, int64_t Q, int
     }
   }
   if (lane == 0) {
-    const float e1 = 1.01f * pair_eps(q_resid[q], __uint_as_float(bank_stats[0]));
+    const float e1 = 1.01f * pair_eps(q_resid[q], __uint_as_float(bank_stats[0]), e_acc);
     float spec = -INFINITY;
     if (T != 0u) {
       const float thr = ord2f(T) - 2.f * e1;
@@ -703,12 +730,12 @@ __global__ void __launch_bounds__(128)
 export_bound_kernel(const uint2* __restrict__ cand, const int* __restrict__ cand_cnt, int SS, int cap, int k,
                     const uint32_t* __restrict__ gthr, int64_t Q, const float* __restrict__ q_resid,
                     const uint32_t* __restrict__ bank_stats, float* __restrict__ bound, int k_part,
-                    float* __restrict__ bound_part) {
+                    float* __restrict__ bound_part, float e_acc) {
   __shared__ uint32_t keys[4][KB_MAX];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t q = (int64_t)blockIdx.x * 4 + warp;
   if (q >= Q) return;
-  const float e1 = 1.01f * pair_eps(q_resid[q], __uint_as_float(bank_stats[0]));
+  const float e1 = 1.01f * pair_eps(q_resid[q], __uint_as_float(bank_stats[0]), e_acc);
   float b = -INFINITY;
   const uint32_t gk = gthr[q];
   if (gk != 0u) {                      // threshold = (lower bound of the k-th best score) - 2.02 eps
@@ -770,12 +797,12 @@ __global__ void fill_kernel(float* __restrict__ x, int64_t n, float v) {
 // running threshold may start there.
 __global__ void __launch_bounds__(256)
 apply_bound_kernel(const float* __restrict__ bound, int64_t Q, const float* __restrict__ q_resid,
-                   const uint32_t* __restrict__ bank_stats, uint32_t* __restrict__ gthr) {
+                   const uint32_t* __restrict__ bank_stats, uint32_t* __restrict__ gthr, float e_acc) {
   const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= Q) return;
   const float b = bound[q];
   if (!(b > -INFINITY) || !(b < INFINITY)) return;
-  const float thr = b - 1.01f * pair_eps(q_resid[q], __uint_as_float(bank_stats[0]));
+  const float thr = b - 1.01f * pair_eps(q_resid[q], __uint_as_float(bank_stats[0]), e_acc);
   if (thr == thr && thr > -INFINITY) {
     const uint32_t key = f2ord(thr);
     if (key > gthr[q]) gthr[q] = key;
@@ -800,42 +827,50 @@ struct RerankParams {
   float* out_dist; int dist_p;     // optional: L1 (p=1) / L2 (p=2) distance of each winner to the raw query
   int* fb_list; int* counters;     // counters[0] = fallback count, [1] = resolved here
   int allow_partial;               // an external bound was applied: fewer than k survivors is legitimate
+  float e_acc;                     // accumulation bound of this width (pair_eps); sits in padding
   const float* spec;               // speculative start threshold per query (NaN / -inf: none)
 };
 
 // exact cosine of one bank row against the query held in qh[] (raw values as doubles):
-// fp64 dot of the raw fp32 rows / (fp64 norm product), rounded once to fp32.
-template <bool VEC, bool L1>
-__device__ __forceinline__ double row_dot(const float* __restrict__ sp, const double (&qh)[8],
+// fp64 dot of the raw fp32 rows / (fp64 norm product), rounded once to fp32.  VPL values per
+// lane: 8 for dim <= 256, 16 for dim <= 512.
+template <bool VEC, bool L1, int VPL>
+__device__ __forceinline__ double row_dot(const float* __restrict__ sp, const double (&qh)[VPL],
                                           int dim, int lane, float* l1) {
   double acc = 0.0;
-  float v[8];
-  if (VEC) {                       // dim == 256, 16-byte aligned rows: d = 4*lane + 128*h + i
-    const float4 a = __ldg(reinterpret_cast<const float4*>(sp) + lane);
-    const float4 b = __ldg(reinterpret_cast<const float4*>(sp) + 32 + lane);
-    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+  float v[VPL];
+  if (VEC) {                       // dim == 8 * VPL, 16-byte aligned rows: d = 4*lane + 128*h + i
+#pragma unroll
+    for (int h = 0; h < VPL / 4; ++h) {
+      const float4 a = __ldg(reinterpret_cast<const float4*>(sp) + 32 * h + lane);
+      v[4 * h] = a.x; v[4 * h + 1] = a.y; v[4 * h + 2] = a.z; v[4 * h + 3] = a.w;
+    }
   } else {                         // d = lane + 32*t
 #pragma unroll
-    for (int t = 0; t < 8; ++t) {
+    for (int t = 0; t < VPL; ++t) {
       const int d = lane + 32 * t;
       v[t] = d < dim ? __ldg(sp + d) : 0.f;
     }
   }
 #pragma unroll
-  for (int t = 0; t < 8; ++t) acc = fma((double)v[t], qh[t], acc);
+  for (int t = 0; t < VPL; ++t) acc = fma((double)v[t], qh[t], acc);
   if (L1) {                        // (compile-time: predicated off it still cost 10 % of the kernel's issue slots)
     float s = 0.f;
 #pragma unroll
-    for (int t = 0; t < 8; ++t) s += fabsf(v[t] - (float)qh[t]);
+    for (int t = 0; t < VPL; ++t) s += fabsf(v[t] - (float)qh[t]);
     *l1 = s;
   }
   return acc;
 }
 
 constexpr int RR_MIN_BLOCKS = 4;   // 5 (96 registers, 140 B of spills) measured equal: latency is hidden by the 4x unrolled loads
-template <bool VEC, bool WANT_L1>
+// VPL = query values per lane (8: dim <= 256, 16: dim <= 512).  The gather keeps the bytes in
+// flight per warp rather than the row count: 8 rows of 1 KiB or 4 rows of 2 KiB (16 values x 8
+// rows would take 128 registers for the loads alone).
+template <bool VEC, bool WANT_L1, int VPL>
 __global__ void __launch_bounds__(128, RR_MIN_BLOCKS)
 rerank_kernel(const RerankParams p, int warps_per_block, int per_warp_entries) {
+  constexpr int RPI = 64 / VPL;              // rows gathered per step
   extern __shared__ __align__(16) unsigned char rr_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int64_t q = (int64_t)blockIdx.x * warps_per_block + warp;
@@ -860,7 +895,7 @@ rerank_kernel(const RerankParams p, int warps_per_block, int per_warp_entries) {
   // (the k-th best of any subset is a lower bound of the global k-th best) and gathering resumes.
   uint32_t g_key = p.gthr[q];
   const float rs_max = __uint_as_float(p.bank_stats[0]);
-  const float e2 = 2.02f * pair_eps(p.q_resid[q], rs_max);
+  const float e2 = 2.02f * pair_eps(p.q_resid[q], rs_max, p.e_acc);
   auto tighten = [&](int count) -> int {      // radix descent (24 bits) + in-place band compaction
     // the keys are cosines of one narrow range: their leading bits agree (typically 9-10 of them),
     // and the descent starts below that common prefix instead of confirming it bit by bit
@@ -956,39 +991,39 @@ rerank_kernel(const RerankParams p, int warps_per_block, int per_warp_entries) {
     return;
   }
   // ---- exact cosine of every survivor
-  double qh[8];
+  double qh[VPL];
   const double nq = p.q_nrm[q];
   const float* qp = p.query + q * p.ldq;
 #pragma unroll
-  for (int t = 0; t < 8; ++t) {
+  for (int t = 0; t < VPL; ++t) {
     const int d = VEC ? (4 * lane + 128 * (t >> 2) + (t & 3)) : (lane + 32 * t);
     qh[t] = d < p.dim ? (double)__ldg(qp + d) : 0.0;
   }
-  // 8 independent row gathers in flight per warp: the phase is DRAM-latency bound otherwise
+  // RPI independent row gathers in flight per warp: the phase is DRAM-latency bound otherwise
   const double ss_q = nq * nq;
-  for (int i = 0; i < n_s; i += 8) {
-    uint32_t r[8];
-    double acc[8];
-    float l1[8];
+  for (int i = 0; i < n_s; i += RPI) {
+    uint32_t r[RPI];
+    double acc[RPI];
+    float l1[RPI];
 #pragma unroll
-    for (int u = 0; u < 8; ++u) r[u] = (uint32_t)ent[min(i + u, n_s - 1)];
+    for (int u = 0; u < RPI; ++u) r[u] = (uint32_t)ent[min(i + u, n_s - 1)];
 #pragma unroll
-    for (int u = 0; u < 8; ++u)
-      acc[u] = row_dot<VEC, WANT_L1>(p.bank + (int64_t)r[u] * p.ldb, qh, p.dim, lane, &l1[u]);
+    for (int u = 0; u < RPI; ++u)
+      acc[u] = row_dot<VEC, WANT_L1, VPL>(p.bank + (int64_t)r[u] * p.ldb, qh, p.dim, lane, &l1[u]);
 #pragma unroll
-    for (int u = 0; u < 8; ++u) acc[u] = warp_sum(acc[u]);
+    for (int u = 0; u < RPI; ++u) acc[u] = warp_sum(acc[u]);
     if (want_l1) {
 #pragma unroll
-      for (int u = 0; u < 8; ++u) l1[u] = warp_sum(l1[u]);
+      for (int u = 0; u < RPI; ++u) l1[u] = warp_sum(l1[u]);
     }
     __syncwarp();
     double a = acc[0];
     uint32_t rr = r[0];
     float l1v = want_l1 ? l1[0] : 0.f;
 #pragma unroll
-    for (int u = 1; u < 8; ++u)
+    for (int u = 1; u < RPI; ++u)
       if (lane == u) { a = acc[u]; rr = r[u]; if (want_l1) l1v = l1[u]; }
-    if (lane < 8 && i + lane < n_s) {
+    if (lane < RPI && i + lane < n_s) {
       const double ns = p.bank_nrm[rr];
       const float v = (float)(a / (nq * ns));
       ent[i + lane] = ((unsigned long long)f2ord(v) << 32) | (unsigned long long)(0xffffffffu - rr);
@@ -1060,6 +1095,7 @@ int tc_cap_for_k(int k) { return k <= 192 ? 256 : (k <= 896 ? 1024 : 0); }
 void tc_workspace(Arena& a, int64_t n_bank, int64_t n_query, int dim, int top_k, TcWorkspace& w) {
   const int nkb = (dim + 63) / 64;
   w.nkb = nkb;
+  w.e_acc = nkb <= 4 ? E_ACC : E_ACC_WIDE;
   w.q_pad = (int64_t)align_up((size_t)n_query, 128);
   w.n_pad = (int64_t)align_up((size_t)n_bank, ST_BN);
   w.plan = plan_lanes(w.q_pad / 128, w.n_pad / ST_BN, sm_count(), ST_MAX_SLOTS);
@@ -1096,17 +1132,22 @@ int launch_pack_rows(const float* x, int64_t rows, int64_t rows_pad, int64_t ld,
   const int wpb = 8;
   const bool vec = (dim % 8 == 0) && (ld % 4 == 0) && ((uintptr_t)x % 16 == 0);
   const unsigned grid = (unsigned)std::min<int64_t>(ceil_div(rows_pad, wpb), (int64_t)sm_count() * 8 * 4);
-  if (vec) pack_rows_kernel<true><<<grid, wpb * 32, 0, st>>>(x, rows, rows_pad, ld, dim, nkb, packed, nrm, resid, stats);
-  else pack_rows_kernel<false><<<grid, wpb * 32, 0, st>>>(x, rows, rows_pad, ld, dim, nkb, packed, nrm, resid, stats);
+  MCLST_REQUIRE(nkb >= 1 && nkb * 64 <= TC_MAX_DIM, MCLST_ERR_UNSUPPORTED, "pack_rows: %d K blocks", nkb);
+  auto kern = nkb <= 4 ? (vec ? pack_rows_kernel<true, 1> : pack_rows_kernel<false, 1>)
+                       : (vec ? pack_rows_kernel<true, 2> : pack_rows_kernel<false, 2>);
+  kern<<<grid, wpb * 32, 0, st>>>(x, rows, rows_pad, ld, dim, nkb, packed, nrm, resid, stats);
   MCLST_LAUNCH_CHECK();
   return 0;
 }
 
 template <int CAP, SimPass PASS>
 static int launch_lanes(const SimParams& p, const LanePlan& L, cudaStream_t st) {
-  auto kern = sim_topk_lanes_kernel<CAP, PASS>;
-  MCLST_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM));
-  kern<<<(unsigned)L.W, ST_THREADS, ST_SMEM, st>>>(p, L);
+  const bool wide = p.nkb > ST_A_BYTES / TP_SLICE_BYTES;
+  auto kern = wide ? sim_topk_lanes_kernel<CAP, PASS, ST_A_BYTES_WIDE, ST_STAGES_WIDE>
+                   : sim_topk_lanes_kernel<CAP, PASS, ST_A_BYTES, ST_STAGES>;
+  const int smem = wide ? st_smem(ST_A_BYTES_WIDE, ST_STAGES_WIDE) : st_smem(ST_A_BYTES, ST_STAGES);
+  MCLST_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  kern<<<(unsigned)L.W, ST_THREADS, smem, st>>>(p, L);
   MCLST_LAUNCH_CHECK();
   return 0;
 }
@@ -1114,7 +1155,7 @@ static int launch_lanes(const SimParams& p, const LanePlan& L, cudaStream_t st) 
 static SimParams sim_params(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int top_k) {
   SimParams p{};
   p.qpack = w.qpack; p.bpack = w.bpack; p.nkb = w.nkb; p.Q = n_query; p.N = n_bank;
-  p.tiles_total = (int)(w.n_pad / ST_BN); p.k = top_k;
+  p.tiles_total = (int)(w.n_pad / ST_BN); p.k = top_k; p.e_acc = w.e_acc;
   p.q_resid = w.q_resid; p.bank_stats = w.stats; p.cand = w.cand; p.cand_cnt = w.cand_cnt;
   p.gthr = w.gthr;
   return p;
@@ -1159,7 +1200,7 @@ int launch_sim_topk(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int t
   }
   if (phase == 2 && sb && sb->ext_bound) {
     apply_bound_kernel<<<(unsigned)ceil_div(n_query, 256), 256, 0, st>>>(sb->ext_bound, n_query, w.q_resid,
-                                                                        w.stats, w.gthr);
+                                                                        w.stats, w.gthr, w.e_acc);
     MCLST_LAUNCH_CHECK();
   }
   if (seeded && phase != 2) {
@@ -1174,7 +1215,7 @@ int launch_sim_topk(const TcWorkspace& w, int64_t n_bank, int64_t n_query, int t
     const int k_seed = speculate ? spec_rank(top_k, (double)w.n_seed / (double)p.tiles_total) : top_k;
     seed_threshold_kernel<<<(unsigned)ceil_div(n_query, 4), 128, 0, st>>>(
         w.seed, w.n_seed * 8, n_query, k_seed, w.q_resid, w.stats, w.gthr, sb ? std::max(1, sb->k_part) : 1,
-        sb ? sb->bound_k : nullptr, sb ? sb->bound_part : nullptr, k_seed < top_k ? w.spec : nullptr);
+        sb ? sb->bound_k : nullptr, sb ? sb->bound_part : nullptr, k_seed < top_k ? w.spec : nullptr, w.e_acc);
     MCLST_LAUNCH_CHECK();
     if (k_seed >= top_k) MCLST_CUDA(cudaMemsetAsync(w.spec, 0xff, (size_t)w.q_pad * sizeof(float), st));  // NaN: none
   } else if (phase != 2) {
@@ -1199,7 +1240,8 @@ int launch_sim_dump(const TcWorkspace& w, int64_t n_bank, int64_t n_query, float
 }
 
 int launch_apply_bound(const TcWorkspace& w, int64_t n_query, const float* ext_bound, cudaStream_t st) {
-  apply_bound_kernel<<<(unsigned)ceil_div(n_query, 256), 256, 0, st>>>(ext_bound, n_query, w.q_resid, w.stats, w.gthr);
+  apply_bound_kernel<<<(unsigned)ceil_div(n_query, 256), 256, 0, st>>>(ext_bound, n_query, w.q_resid, w.stats, w.gthr,
+                                                                      w.e_acc);
   MCLST_LAUNCH_CHECK();
   return 0;
 }
@@ -1207,7 +1249,8 @@ int launch_export_bound(const TcWorkspace& w, int64_t n_query, int top_k, float*
                         float* bound_part, cudaStream_t st) {
   export_bound_kernel<<<(unsigned)ceil_div(n_query, 4), 128, 0, st>>>(w.cand, w.cand_cnt, w.SS, w.cap, top_k, w.gthr,
                                                                      n_query, w.q_resid, w.stats, bound,
-                                                                     std::max(1, std::min(k_part, top_k)), bound_part);
+                                                                     std::max(1, std::min(k_part, top_k)), bound_part,
+                                                                     w.e_acc);
   MCLST_LAUNCH_CHECK();
   return 0;
 }
@@ -1219,7 +1262,7 @@ int launch_rerank(const TcWorkspace& w, const float* bank, int64_t n_bank, int64
   RerankParams p;
   p.allow_partial = allow_partial ? 1 : 0;
   p.spec = allow_partial ? nullptr : w.spec;
-  p.cand = w.cand; p.cand_cnt = w.cand_cnt; p.SS = w.SS; p.cap = w.cap; p.k = top_k;
+  p.cand = w.cand; p.cand_cnt = w.cand_cnt; p.SS = w.SS; p.cap = w.cap; p.k = top_k; p.e_acc = w.e_acc;
   p.Q = n_query; p.N = n_bank; p.bank = bank; p.ldb = ldb; p.bank_nrm = w.b_nrm;
   p.query = query; p.ldq = ldq; p.q_nrm = w.q_nrm; p.q_resid = w.q_resid;
   p.bank_stats = w.stats; p.q_stats = w.stats + 8; p.gthr = w.gthr; p.dim = dim;
@@ -1234,7 +1277,8 @@ int launch_rerank(const TcWorkspace& w, const float* bank, int64_t n_bank, int64
   int wpb = 4;
   while (wpb > 1 && (size_t)wpb * per_warp * 8 > 64 * 1024) wpb >>= 1;
   const size_t smem = (size_t)wpb * per_warp * 8 + (size_t)wpb * RR_MAX * 6;
-  const bool vec = (dim == 256) && (ldb % 4 == 0) && (ldq % 4 == 0) && ((uintptr_t)bank % 16 == 0) &&
+  const bool wide = dim > 256;
+  const bool vec = (dim == (wide ? 512 : 256)) && (ldb % 4 == 0) && (ldq % 4 == 0) && ((uintptr_t)bank % 16 == 0) &&
                    ((uintptr_t)query % 16 == 0);
   const bool l1 = out_dist != nullptr && dist_p == 1;
   const unsigned grid = (unsigned)ceil_div(n_query, wpb);
@@ -1247,10 +1291,15 @@ int launch_rerank(const TcWorkspace& w, const float* bank, int64_t n_bank, int64
     kern<<<grid, 128, smem, st>>>(p, wpb, per_warp);
     return 0;
   };
-  static size_t attr[4] = {0, 0, 0, 0};
+  static size_t attr[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   int rc;
-  if (vec) rc = l1 ? launch(rerank_kernel<true, true>, attr[3]) : launch(rerank_kernel<true, false>, attr[2]);
-  else rc = l1 ? launch(rerank_kernel<false, true>, attr[1]) : launch(rerank_kernel<false, false>, attr[0]);
+  if (wide) {
+    if (vec) rc = l1 ? launch(rerank_kernel<true, true, 16>, attr[7]) : launch(rerank_kernel<true, false, 16>, attr[6]);
+    else rc = l1 ? launch(rerank_kernel<false, true, 16>, attr[5]) : launch(rerank_kernel<false, false, 16>, attr[4]);
+  } else {
+    if (vec) rc = l1 ? launch(rerank_kernel<true, true, 8>, attr[3]) : launch(rerank_kernel<true, false, 8>, attr[2]);
+    else rc = l1 ? launch(rerank_kernel<false, true, 8>, attr[1]) : launch(rerank_kernel<false, false, 8>, attr[0]);
+  }
   if (rc) return rc;
   MCLST_LAUNCH_CHECK();
   return 0;

@@ -165,8 +165,9 @@ def _all_gather_cat(t: torch.Tensor, group, async_op: bool = False):
 
 
 def _tc_eligible(shard: BankShard, k: int) -> bool:
+    from .retrieval import tc_eligible
     n, d = shard.spot_key.shape
-    return d <= 256 and k <= 896 and n >= k
+    return tc_eligible(n, d, k)
 
 
 class _Block:

@@ -26,7 +26,7 @@ ArrayLike = Union[np.ndarray, torch.Tensor]
 __all__ = ["find_matches", "find_matches_cscc", "find_matches_device", "fm_workspace", "fm_pack_bank", "fm_seed",
            "fm_candidates", "fm_main", "weighted_topk_average",
            "weighted_topk_average_device", "retrieve", "retrieve_device", "retrieve_workspace", "last_counters",
-           "to_host", "Bank"]
+           "to_host", "tc_eligible", "Bank"]
 
 _last_ws: Optional[torch.Tensor] = None
 _side_streams: dict = {}
@@ -81,6 +81,13 @@ def _dev_f32(x: ArrayLike, device=None) -> torch.Tensor:
     if t.stride(-1) != 1:
         t = t.contiguous()
     return t
+
+
+def tc_eligible(n_bank: int, dim: int, top_k: int, flags: int = _lib.FM_DEFAULT) -> bool:
+    """Whether find_matches of this shape runs the tensor-core candidate pass (and a bank of it can
+    keep a packed image) or brute-forces every query: the library's own rule
+    (mclst_find_matches_tc_eligible), asked rather than restated.  Needs no GPU."""
+    return bool(load().mclst_find_matches_tc_eligible(int(n_bank), int(dim), int(top_k), int(flags)))
 
 
 def find_matches_device(spot_embeddings: torch.Tensor, query_embeddings: torch.Tensor,
@@ -419,8 +426,7 @@ class Bank:
     def find_matches(self, query: torch.Tensor, top_k: int = 50, dist_p: Optional[int] = None):
         """Device-resident (values, indices[, distances]) against the resident packed image."""
         N, D = self.spot_key.shape
-        eligible = D <= 256 and top_k <= 896 and N >= top_k
-        if not eligible or query.shape[0] == 0:
+        if not tc_eligible(N, D, top_k) or query.shape[0] == 0:
             return find_matches_device(self.spot_key, query, top_k, dist_p=dist_p)
         ws = self._workspace(query.shape[0], top_k)
         fm_seed(self.spot_key, query, top_k, ws, bank_packed=True)
@@ -430,7 +436,7 @@ class Bank:
     def retrieve_device(self, image_query: torch.Tensor, top_k: int = 50, mode: str = "inv_sq_l2",
                         want_emb: bool = False, out_dtype=torch.float32):
         N, D = self.spot_key.shape
-        if D <= 256 and top_k <= 896 and N >= top_k and image_query.shape[0] > 0:
+        if tc_eligible(N, D, top_k) and image_query.shape[0] > 0:
             ws = self._workspace(image_query.shape[0], top_k)
             return _retrieve_call(self.spot_key, self.expression_key, image_query, top_k, mode, want_emb,
                                   out_dtype, _lib.FM_BANK_PACKED, ws)
